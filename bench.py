@@ -204,6 +204,8 @@ def main():
     ap.add_argument("--baseline-timeout", type=int, default=200)
     ap.add_argument("--no-block-grad", action="store_true", help="A/B: block-gradient merge as separate reduce passes")
     ap.add_argument("--stem-bwd-fuse", action="store_true", help="A/B (opt-in): max-pool backward fused with the stem-BN backward")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last step computed as "
+                                                         "DIR/<name>.npy (rank 0), to compare two builds output for output")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
 
@@ -272,6 +274,8 @@ def main():
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
     ms = float(dist.allreduce(ms, average=False).item()) if world == 1 else float(_max_over_ranks(ms))
     loss, acc = step.result()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, engine, loss, acc)
     # outside the timed region: after K data-parallel steps every rank must hold bit-identical fp32 master weights
     # (a gradient that was all-reduced before its producer finished would show up here)
     from b200ddl.utils import checksum_across_ranks
@@ -352,6 +356,32 @@ def main():
         print(json.dumps(out), flush=True)
     dist.shutdown()
     return 0
+
+
+DUMP_WEIGHT_SAMPLE = 1 << 22   # 16 MB of the 25.6 M fp32 weights (102 MB): the dump stays far below 64 MB
+
+
+def dump_outputs(out_dir: str, engine, loss: float, acc: float) -> None:
+    """Write what a training step hands its caller, as it stands after the last timed step: loss and accuracy, the fp32
+    logits, the BatchNorm running statistics and a fixed, seeded sample of the updated fp32 weights.  Tensors are taken
+    in torchvision names and layouts and concatenated in name order, so two builds compare element for element even
+    when their internal parameter layouts differ.  Compare with a tolerance: the reductions use floating-point atomics,
+    so two runs of one build already differ after a few dozen training steps."""
+    import numpy as np
+    import torch
+
+    sd = engine.state_dict()
+    stats = sorted(k for k in sd if k.endswith((".running_mean", ".running_var")))
+    weights = sorted(set(sd) - set(stats))
+    w = torch.cat([sd[k].reshape(-1) for k in weights]).numpy()
+    idx = np.sort(np.random.default_rng(0).choice(w.size, min(DUMP_WEIGHT_SAMPLE, w.size), replace=False))
+    arrays = {"loss": np.array([loss], np.float64), "accuracy": np.array([acc], np.float64),
+              "logits": engine.logits.float().cpu().numpy(),
+              "bn_running_stats": torch.cat([sd[k].reshape(-1) for k in stats]).numpy(),
+              "weights_sample": w[idx]}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def _max_over_ranks(t):

@@ -81,7 +81,8 @@ def test_parallel_trials_run_concurrently(tmp_path):
             cur[0] -= 1
         return p["x"] ** 2
 
-    t = ParallelTrials(parallelism=4)
+    # threads: the objective counts its concurrency in this process ('auto' picks worker processes on a GPU machine)
+    t = ParallelTrials(parallelism=4, executor="thread")
     fmin(obj, {"x": hp.uniform("x", -1, 1)}, algo=tpe.suggest, max_evals=16, trials=t, rstate=0)
     assert len(t) == 16 and 2 <= peak[0] <= 4
 
@@ -152,7 +153,8 @@ def test_hyperopt_stopping_arguments():
     t = Trials()
     fmin(lambda p: 1.0, space, algo=rand.suggest, max_evals=200, trials=t, rstate=2, early_stop_fn=no_progress)
     assert len(t) == 6                                      # first trial sets the best, five stale ones follow
-    t = ParallelTrials(parallelism=4)
+    # threads: a 0.5 s budget is shorter than starting the worker processes 'auto' picks on a GPU machine
+    t = ParallelTrials(parallelism=4, executor="thread")
     fmin(lambda p: (time.sleep(0.05), p["x"] ** 2)[1], space, algo=rand.suggest, max_evals=1000, trials=t, rstate=3, timeout=0.5)
     assert 4 <= len(t) < 120 and all(tr["result"].get("status") == STATUS_OK for tr in t.trials)
     with pytest.warns(UserWarning):

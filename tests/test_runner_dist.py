@@ -188,8 +188,11 @@ def test_workers_get_their_share_of_the_cores(monkeypatch):
         hvd.init()
         return os.environ.get("OMP_NUM_THREADS"), torch.get_num_threads()
 
+    from b200ddl.utils.cpus import usable_cpus
+
     monkeypatch.delenv("OMP_NUM_THREADS", raising=False)
-    share = max(1, (os.cpu_count() or 1) // 2)
+    monkeypatch.delenv("MKL_NUM_THREADS", raising=False)   # torch sizes its team from MKL_NUM_THREADS when that is set
+    share = max(1, usable_cpus() // 2)
     env_val, torch_threads = Runner(np=2, driver_log_verbosity="none", force_cpu=True).run(fn)
     assert env_val == str(share) and torch_threads == share
     monkeypatch.setenv("OMP_NUM_THREADS", "3")           # an explicit user setting wins

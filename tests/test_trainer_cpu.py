@@ -19,10 +19,10 @@ def make_ds(batch=8, size=32, classes=5, seed=0):
 
 
 def test_reference_model_only_head_is_trainable():
-    m = build_model(224, 224, 3, 5, arch="mobilenetv2")
+    m = build_model(224, 224, 3, 5, arch="mobilenetv2", device="cpu")   # the torch module, also where a GPU exists
     trainable = sum(p.numel() for p in m.parameters() if p.requires_grad)
     assert trainable == 1280 * 5 + 5 == 6405                       # SURVEY.md Q11 / P1/03:168-169
-    assert build_model(0.3, arch="mobilenetv2").dropout.p == 0.3    # build_model(dropout) form (P2/01:92)
+    assert build_model(0.3, arch="mobilenetv2", device="cpu").dropout.p == 0.3    # build_model(dropout) form (P2/01:92)
 
 
 def test_fit_evaluate_predict_history_and_callbacks(tmp_path):
@@ -67,7 +67,7 @@ def test_autolog_and_model_reload(tmp_path):
     tracking.set_experiment("e")
     tracking.autolog()
     try:
-        model = build_model(32, 32, 3, 5, arch="mobilenetv2")
+        model = build_model(32, 32, 3, 5, arch="mobilenetv2", device="cpu")
         tr = Trainer(model, device="cpu").compile(optimizer=optim.Adam(1e-3))
         with tracking.start_run(run_name="single_node") as run:
             tr.fit(make_ds(), steps_per_epoch=2, epochs=2, verbose=0, validation_data=make_ds(seed=2), validation_steps=1)
@@ -122,7 +122,7 @@ def test_save_load_resume_continues_training(tmp_path):
     x = np.zeros((2, 32, 32, 3), np.uint8)
     assert np.allclose(a.predict(x), c.predict(x), atol=1e-5)
     # optimizer mismatch is an error, not silent garbage
-    d = Trainer(build_model(32, 32, 3, 5, arch="mobilenetv2"), device="cpu").compile(optimizer=optim.SGD(0.1))
+    d = Trainer(build_model(32, 32, 3, 5, arch="mobilenetv2", device="cpu"), device="cpu").compile(optimizer=optim.SGD(0.1))
     with pytest.raises(ValueError):
         d.load(path)
 
