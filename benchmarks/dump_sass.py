@@ -23,10 +23,10 @@ COUNT = [("UTCHMMA", r"\bUTCHMMA\b"), ("UTMALDG", r"\bUTMALDG"), ("UTMASTG", r"\
 # substrings of demangled names whose full listing is written out
 SELECT = ["conv_igemm_kernel<64, 1, true, true>", "conv_igemm_kernel<64, 2, true, true>", "conv_igemm_kernel<256, 1, false, false>",
           "conv_igemm_kernel<256, 2, false, false>", "conv_igemm_kernel<256, 3, false, false>", "conv_igemm_kernel<256, 4, false, false>",
-          "allreduce_twoshot_nvls_kernel<(b200::CommDtype)0, 8>", "broadcast_kernel<(b200::CommDtype)0>", "stem_pool_bn_bwd_kernel<0>",
+          "allreduce_twoshot_nvls_kernel<(b200::CommDtype)0, 8>", "broadcast_kernel<(b200::CommDtype)0>",
           "softmax_ce_head_kernel", "dwconv3x3_kernel<1>", "dwconv3x3_tiled_kernel<1, 4>", "resize_triangle_batched_kernel", "mbv2_stem_kernel", "weight_prep_batched_kernel", "conv_wgrad_kernel", "stem_fwd_kernel", "stem_wgrad_kernel",
           "allreduce_twoshot_nvls_kernel<(b200::CommDtype)0", "allreduce_sgd_nvls_kernel", "allreduce_twoshot_p2p_kernel<(b200::CommDtype)0, 2>",
-          "bn_apply_kernel<true, 1, false, 1>", "col_reduce_kernel<4>", "bn_bwd_apply_kernel<true, false, 1>", "sgd_kernel<false>",
+          "bn_apply_kernel<true, 1>", "col_reduce_kernel<4>", "bn_bwd_apply_kernel<true>", "sgd_kernel<false>",
           "adam_kernel", "softmax_ce_kernel", "bn_relu_maxpool_fwd_kernel", "tma_probe_kernel", "umma_probe_kernel"]
 
 

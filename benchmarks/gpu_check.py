@@ -236,50 +236,6 @@ def case_elementwise():
         yr3 = yf.clone().requires_grad_(True)
         torch.nn.functional.batch_norm(yr3, None, None, gamma, beta, True, 0.1, 1e-5).backward(gout.float())
         ok &= report(f"bn_bwd_dy_mode3/C{C_}", rel_err(dy3, yr3.grad), 2e-2)
-        # ---- fused coefficient variants: same results as finalize + apply / coeffs + apply without the tiny launches
-        def fresh_pack(src, ga, be):
-            s_ = torch.zeros(C_, device=DEV); q_ = torch.zeros(C_, device=DEV)
-            e.channel_stats(src, s_, q_)
-            return [s_, q_, ga, be, torch.zeros(C_, device=DEV), torch.ones(C_, device=DEV), torch.empty(C_, device=DEV),
-                    torch.empty(C_, device=DEV), torch.empty(C_, device=DEV), torch.empty(C_, device=DEV)]
-
-        pk = fresh_pack(y, gamma, beta)
-        out_f = torch.empty_like(y)
-        mask_f = torch.zeros(M * C_ // 8, device=DEV, dtype=torch.uint8)
-        e.bn_apply_fused(y, pk, float(M), 0.1, 1e-5, res, None, out_f, True, mask_f)
-        ok &= report(f"bn_apply_fused_out/C{C_}", rel_err(out_f, out), 4e-3, f"mismatching elements {float((out_f != out).float().mean()):.2e}")
-        ok &= report(f"bn_apply_fused_mask/C{C_}", float((mask_f != mask).float().mean()), 1e-4)
-        for nm, a_, b_ in (("mean", pk[6], mean), ("invstd", pk[7], invstd), ("scale", pk[8], scale), ("shift", pk[9], shift),
-                           ("running_mean", pk[4], rm), ("running_var", pk[5], rv)):
-            ok &= report(f"bn_apply_fused_{nm}/C{C_}", rel_err(a_, b_), 2e-6)
-        ok &= report(f"bn_apply_fused_sums_untouched/C{C_}", float(pk[0].abs().max() == 0), 0.0)
-        # residual with its own BatchNorm (downsample branch)
-        gamma_r = torch.rand(C_, device=DEV, generator=g) + 0.5
-        beta_r = torch.randn(C_, device=DEV, generator=g)
-        pk_m, pk_r = fresh_pack(y, gamma, beta), fresh_pack(res, gamma_r, beta_r)
-        out_f2 = torch.empty_like(y)
-        e.bn_apply_fused(y, pk_m, float(M), 0.1, 1e-5, res, pk_r, out_f2, True, None)
-        sr = torch.zeros(C_, device=DEV); qr = torch.zeros(C_, device=DEV)
-        e.channel_stats(res, sr, qr)
-        r_mean = torch.empty(C_, device=DEV); r_is = torch.empty(C_, device=DEV)
-        r_scale = torch.empty(C_, device=DEV); r_shift = torch.empty(C_, device=DEV)
-        e.bn_finalize(sr, qr, float(M), gamma_r, beta_r, torch.zeros(C_, device=DEV), torch.ones(C_, device=DEV), 0.1, 1e-5,
-                      r_mean, r_is, r_scale, r_shift, True)
-        out_u2 = torch.empty_like(y)
-        e.bn_apply(y, scale, shift, res, r_scale, r_shift, out_u2, True)
-        ok &= report(f"bn_apply_fused_bn_residual/C{C_}", rel_err(out_f2, out_u2), 4e-3)
-        ok &= report(f"bn_apply_fused_res_scale/C{C_}", rel_err(pk_r[8], r_scale), 2e-6)
-        # backward: A, B, C in the apply prologue, dgamma / dbeta written by the kernel
-        s2 = torch.zeros(C_, device=DEV); s2y = torch.zeros(C_, device=DEV)
-        e.bn_bwd_reduce(2, gout, None, None, y, scale, shift, None, s2, s2y)
-        dg_f = torch.empty(C_, device=DEV); db_f = torch.empty(C_, device=DEV); dy_f = torch.empty_like(y)
-        e.bn_bwd_apply_fused(gout, y, scale, shift, s2, s2y, gamma, mean, invstd, float(M), dg_f, db_f, dy_f)
-        dg_u = torch.empty(C_, device=DEV); db_u = torch.empty(C_, device=DEV); dy_u = torch.empty_like(y)
-        e.bn_bwd_coeffs(s2, s2y, gamma, mean, invstd, float(M), dg_u, db_u, cA, cB, cC)
-        e.bn_bwd_apply(gout, y, scale, shift, cA, cB, cC, dy_u)
-        ok &= report(f"bn_bwd_apply_fused_dy/C{C_}", rel_err(dy_f, dy_u), 4e-3)
-        ok &= report(f"bn_bwd_apply_fused_dgamma/C{C_}", rel_err(dg_f, dg_u), 2e-6)
-        ok &= report(f"bn_bwd_apply_fused_dbeta/C{C_}", rel_err(db_f, db_u), 2e-6)
         # autograd reference
         yr = yf.clone().requires_grad_(True)
         gr = gamma.clone().requires_grad_(True); br = beta.clone().requires_grad_(True)
@@ -341,12 +297,6 @@ def case_elementwise():
         ok &= report(f"softmax_ce_grad/K{K}", rel_err(dl, lg.grad), 1e-3)
         acc = (logits.argmax(1) == labels).float().sum().item()
         ok &= report(f"softmax_ce_acc/K{K}", abs(st[1].item() - acc), 0.0)
-    # preprocess
-    xb = torch.randint(0, 256, (2, 32, 32, 3), device=DEV, dtype=torch.uint8, generator=g)
-    ob = torch.empty(2, 32, 32, 8, device=DEV, dtype=torch.bfloat16)
-    e.preprocess_u8(xb, ob, 1 / 127.5, -1.0)
-    ok &= report("preprocess_u8", rel_err(ob[..., :3], xb.float() / 127.5 - 1), 1e-2)
-    ok &= report("preprocess_u8_pad", float(ob[..., 3:].float().abs().max()), 0.0)
     # bilinear resize (half-pixel centres, no antialias - tf.image.resize / F.interpolate(align_corners=False))
     for (H_, W_, OH, OW) in ((64, 48, 32, 32), (40, 40, 96, 96), (224, 224, 224, 224)):
         xs = torch.randint(0, 256, (3, H_, W_, 3), device=DEV, dtype=torch.uint8, generator=g)
@@ -438,7 +388,7 @@ def case_conv_time():
     return True
 
 
-def case_engine(overlap_wgrad: bool = True, quick: bool = False, fuse_bn_coeffs: bool = False, fuse_block_grad=None):
+def case_engine(overlap_wgrad: bool = True, quick: bool = False, fuse_block_grad=None):
     """ResNet-50 engine forward/backward vs torchvision (same weights, fp32 reference and bf16-autocast reference).
 
     `overlap_wgrad` selects where the weight-gradient GEMMs are issued (side stream = the engine default, or in line);
@@ -450,9 +400,9 @@ def case_engine(overlap_wgrad: bool = True, quick: bool = False, fuse_bn_coeffs:
     ok = True
     N, K = 32, 10
     eng = ResNet50Engine(batch=N, num_classes=K, zero_init_residual=False, seed=1, overlap_wgrad=overlap_wgrad,
-                         fuse_bn_coeffs=fuse_bn_coeffs, fuse_block_grad=fuse_block_grad)
+                         fuse_block_grad=fuse_block_grad)
     print(f"INFO engine overlap_wgrad={eng.overlap_wgrad} fuse_bwd_reduce={eng.fuse_bwd_reduce} "
-          f"fuse_bn_coeffs={eng.fuse_bn_coeffs} fuse_block_grad={eng.fuse_block_grad} fuse_stem_bwd={eng.fuse_stem_bwd}", flush=True)
+          f"fuse_block_grad={eng.fuse_block_grad}", flush=True)
     opt = optim.SGD(learning_rate=0.1, momentum=0.9)
     step = EngineTrainStep(eng, opt, use_graph=False)
     g = torch.Generator(device=DEV).manual_seed(5)
@@ -762,71 +712,6 @@ def case_head():
     return ok
 
 
-def case_stem_bwd():
-    """max-pool backward fused with the stem BN+ReLU backward (head_stem.cu) vs the three-kernel path it replaces."""
-    ok = True
-    e = ops.ext("_b200_ops")
-    for N, Ho in ((4, 16), (3, 56), (256, 56)):
-        g = torch.Generator(device=DEV).manual_seed(31)
-        H = 2 * Ho
-        y0 = torch.randn(N, H, H, 64, device=DEV, generator=g).to(torch.bfloat16)
-        scale = torch.rand(64, device=DEV, generator=g) + 0.5
-        shift = torch.randn(64, device=DEV, generator=g) * 0.3
-        p0 = torch.empty(N, Ho, Ho, 64, device=DEV, dtype=torch.bfloat16)
-        idx = torch.empty(N, Ho, Ho, 64, device=DEV, dtype=torch.uint8)
-        e.bn_relu_maxpool_fwd(y0, scale, shift, p0, idx)
-        g1 = torch.randn(N, Ho, Ho, 64, device=DEV, generator=g).to(torch.bfloat16)
-        g2 = torch.randn(N, Ho, Ho, 64, device=DEV, generator=g).to(torch.bfloat16)
-        gamma = torch.rand(64, device=DEV, generator=g) + 0.5
-        mean = torch.randn(64, device=DEV, generator=g) * 0.1
-        invstd = torch.rand(64, device=DEV, generator=g) + 0.5
-        cnt = float(N * H * H)
-        # old path
-        da0 = torch.empty_like(y0)
-        e.maxpool_bwd(idx, g1, g2, da0)
-        s_o = torch.zeros(64, device=DEV); sy_o = torch.zeros(64, device=DEV)
-        e.bn_bwd_reduce(2, da0, None, None, y0, scale, shift, None, s_o, sy_o)
-        s_keep, sy_keep = s_o.clone(), sy_o.clone()
-        dg = torch.empty(64, device=DEV); db = torch.empty(64, device=DEV)
-        cA = torch.empty(64, device=DEV); cB = torch.empty(64, device=DEV); cC = torch.empty(64, device=DEV)
-        e.bn_bwd_coeffs(s_o, sy_o, gamma, mean, invstd, cnt, dg, db, cA, cB, cC)
-        dy_o = torch.empty_like(y0)
-        e.bn_bwd_apply(da0, y0, scale, shift, cA, cB, cC, dy_o)
-        # fused path
-        s_n = torch.zeros(64, device=DEV); sy_n = torch.zeros(64, device=DEV)
-        e.stem_pool_bn_bwd(0, idx, g1, g2, y0, scale, shift, None, None, None, None, s_n, sy_n)
-        dy_n = torch.full_like(y0, 7.0)
-        e.stem_pool_bn_bwd(1, idx, g1, g2, y0, scale, shift, cA, cB, cC, dy_n, s_n, sy_n)
-        torch.cuda.synchronize()
-        ok &= report(f"stem_bwd_sum_dz/N{N}_Ho{Ho}", float((s_n - s_keep).abs().max() / (s_keep.abs().max() + 1e-6)), 1e-4)
-        ok &= report(f"stem_bwd_sum_dzy/N{N}_Ho{Ho}", float((sy_n - sy_keep).abs().max() / (sy_keep.abs().max() + 1e-6)), 1e-4)
-        # the scatter sums the <= 4 window contributions of a pixel in colour-class order, the unfused kernel in window
-        # order: fp32 sums may differ in the last bit, i.e. rarely one bf16 ulp after rounding
-        mism = float((dy_n != dy_o).float().mean())
-        ok &= report(f"stem_bwd_dy/N{N}_Ho{Ho}", rel_err(dy_n, dy_o), 8e-3, f"(vs the unfused path; differing elements {mism:.2e})")
-        ok &= report(f"stem_bwd_dy_mismatch_rate/N{N}_Ho{Ho}", mism, 2e-3)
-        # one-gradient variant (g2 = None)
-        e.maxpool_bwd(idx, g1, None, da0)
-        e.bn_bwd_apply(da0, y0, scale, shift, cA, cB, cC, dy_o)
-        e.stem_pool_bn_bwd(1, idx, g1, None, y0, scale, shift, cA, cB, cC, dy_n, s_n, sy_n)
-        torch.cuda.synchronize()
-        ok &= report(f"stem_bwd_dy_single_grad/N{N}_Ho{Ho}", rel_err(dy_n, dy_o), 8e-3)
-        if N >= 256:
-            flush = torch.empty(256 * 1024 * 1024, device=DEV, dtype=torch.uint8)
-            def old():
-                e.maxpool_bwd(idx, g1, g2, da0)
-                e.bn_bwd_reduce(2, da0, None, None, y0, scale, shift, None, s_o, sy_o)
-                e.bn_bwd_apply(da0, y0, scale, shift, cA, cB, cC, dy_o)
-            def new():
-                e.stem_pool_bn_bwd(0, idx, g1, g2, y0, scale, shift, None, None, None, None, s_n, sy_n)
-                e.stem_pool_bn_bwd(1, idx, g1, g2, y0, scale, shift, cA, cB, cC, dy_n, s_n, sy_n)
-            t_o = time_fn(old, flush=flush); t_n = time_fn(new, flush=flush)
-            t_r = time_fn(lambda: e.stem_pool_bn_bwd(0, idx, g1, g2, y0, scale, shift, None, None, None, None, s_n, sy_n), flush=flush)
-            print(f"TIME stem_bwd N{N}: unfused (pool_bwd+reduce+apply)={t_o*1e3:.0f}us fused (reduce+apply)={t_n*1e3:.0f}us "
-                  f"[reduce pass {t_r*1e3:.0f}us]", flush=True)
-    return ok
-
-
 def case_big_numerics():
     """Numerics at the BENCHMARKED shapes (batch 256: full grids, halo / resident-filter paths, 802,816-pixel M) vs fp32."""
     ok = True
@@ -1062,72 +947,6 @@ def case_mobilenet():
 
 
 
-def case_tails():
-    """Last-CTA tails of the conv kernels: BatchNorm finalize after a forward GEMM with statistics, backward coefficients
-    after a dgrad GEMM with the fused reduction - vs the stand-alone bn_finalize / bn_bwd_coeffs kernels, run twice
-    (the ticket counter and the sums must be back at zero, as a CUDA-graph replay needs)."""
-    ok = True
-    e = ops.ext("_b200_ops")
-    g = torch.Generator(device=DEV).manual_seed(61)
-    for name, N, H, W, cin, cout, R, stride, pad in [s_ for s_ in CONV_SHAPES if s_[0] in ("1x1_64_256_56", "3x3_64_64_56", "3x3_256_256_14", "1x1_512_2048_7", "3x3s2_128_128_56")]:
-        x, w, Ho, Wo = make_conv_case(N, H, W, cin, cout, R, stride, pad)
-        wk = w.to(torch.bfloat16).reshape(R * R * cout, cin).contiguous()
-        y = torch.empty(N, Ho, Wo, cout, device=DEV, dtype=torch.bfloat16)
-        ssum = torch.zeros(cout, device=DEV); ssq = torch.zeros(cout, device=DEV)
-        gamma = torch.rand(cout, device=DEV, generator=g) + 0.5; beta = torch.randn(cout, device=DEV, generator=g)
-        rm = torch.zeros(cout, device=DEV); rv = torch.ones(cout, device=DEV)
-        outs = [torch.empty(cout, device=DEV) for _ in range(4)]
-        ctr = torch.zeros(1, device=DEV, dtype=torch.int32)
-        op = C.ConvForward(x, wk, y, R, R, stride, pad, ssum, ssq)
-        cnt = float(N * Ho * Wo)
-        op.plan.set_bn_finalize(ctr, gamma, beta, rm, rv, outs[0], outs[1], outs[2], outs[3], cnt, 0.1, 1e-5)
-        for rep in range(2):
-            op.run()
-        torch.cuda.synchronize()
-        # reference: statistics of the bf16 output, through the stand-alone kernel, applied twice to the running stats
-        s2 = torch.zeros(cout, device=DEV); q2 = torch.zeros(cout, device=DEV)
-        rm2 = torch.zeros(cout, device=DEV); rv2 = torch.ones(cout, device=DEV)
-        ref = [torch.empty(cout, device=DEV) for _ in range(4)]
-        for rep in range(2):
-            e.channel_stats(y, s2, q2)
-            e.bn_finalize(s2, q2, cnt, gamma, beta, rm2, rv2, 0.1, 1e-5, ref[0], ref[1], ref[2], ref[3], True)
-        torch.cuda.synchronize()
-        for nm, a_, b_ in (("mean", outs[0], ref[0]), ("invstd", outs[1], ref[1]), ("scale", outs[2], ref[2]), ("shift", outs[3], ref[3]),
-                           ("running_mean", rm, rm2), ("running_var", rv, rv2)):
-            ok &= report(f"tail_finalize_{nm}/{name}", float((a_ - b_).abs().max() / (b_.abs().max() + 1e-6)), 2e-3)
-        ok &= report(f"tail_finalize_sums_zeroed/{name}", float(ssum.abs().max() + ssq.abs().max() + ctr.abs().sum()), 0.0)
-        op.plan.enable_tail(False)   # eval mode: sums stay, nothing is finalized
-        before = outs[0].clone()
-        op.run(); torch.cuda.synchronize()
-        ok &= report(f"tail_disabled_keeps_sums/{name}", float(ssum.abs().max() == 0) + float((outs[0] - before).abs().max()), 0.0)
-        ssum.zero_(); ssq.zero_()
-        if stride == 1:
-            dy = torch.randn(N, Ho, Wo, cout, device=DEV, generator=g).to(torch.bfloat16)
-            yb = torch.randn(N, H, W, cin, device=DEV, generator=g).to(torch.bfloat16)
-            sc = torch.rand(cin, device=DEV, generator=g) + 0.5; sh = torch.randn(cin, device=DEV, generator=g) * 0.5
-            s_dz = torch.zeros(cin, device=DEV); s_dzy = torch.zeros(cin, device=DEV)
-            dx = torch.empty(N, H, W, cin, device=DEV, dtype=torch.bfloat16)
-            gam = torch.rand(cin, device=DEV, generator=g) + 0.5
-            mean = torch.randn(cin, device=DEV, generator=g) * 0.1; invstd = torch.rand(cin, device=DEV, generator=g) + 0.5
-            o = [torch.empty(cin, device=DEV) for _ in range(5)]
-            ctr2 = torch.zeros(1, device=DEV, dtype=torch.int32)
-            dg = C.ConvDgrad(dy, w, dx, R, R, stride, pad, bwd_stats=(yb, sc, sh, s_dz, s_dzy))
-            cnt2 = float(N * H * W)
-            dg.parts[0][0].set_bn_bwd_coeffs(ctr2, gam, mean, invstd, cnt2, o[0], o[1], o[2], o[3], o[4])
-            for rep in range(2):
-                dg.run()
-            torch.cuda.synchronize()
-            s3 = torch.zeros(cin, device=DEV); q3 = torch.zeros(cin, device=DEV)
-            e.bn_bwd_reduce(2, dx, None, None, yb, sc, sh, None, s3, q3)
-            r = [torch.empty(cin, device=DEV) for _ in range(5)]
-            e.bn_bwd_coeffs(s3, q3, gam, mean, invstd, cnt2, r[0], r[1], r[2], r[3], r[4])
-            torch.cuda.synchronize()
-            for nm, a_, b_ in zip(("dgamma", "dbeta", "cA", "cB", "cC"), o, r):
-                ok &= report(f"tail_bwd_{nm}/{name}", float((a_ - b_).abs().max() / (b_.abs().max() + 1e-6)), 3e-3)
-            ok &= report(f"tail_bwd_sums_zeroed/{name}", float(s_dz.abs().max() + s_dzy.abs().max() + ctr2.abs().sum()), 0.0)
-    return ok
-
-
 def case_umma_probe():
     """Row-shifted SWIZZLE_128B descriptors: which (shift, base_offset) combinations read the right rows?"""
     ext = ops.ext("_b200_probe")
@@ -1213,15 +1032,12 @@ CASES = {
     "engine": case_engine,
     "tma_probe": case_tma_probe,
     "engine_serial_wgrad": lambda: case_engine(overlap_wgrad=False, quick=True),
-    "engine_fused_bn_coeffs": lambda: case_engine(quick=True, fuse_bn_coeffs=True),
     "stem": case_stem,
     "block_grad": case_block_grad,
     "head": case_head,
-    "stem_bwd": case_stem_bwd,
     "big_numerics": case_big_numerics,
     "fused_infer": case_fused_infer,
     "mobilenet": case_mobilenet,
-    "tails": case_tails,
     "engine_unfused_block_grad": lambda: case_engine(quick=True, fuse_block_grad=False),
     "umma_probe": case_umma_probe,
 }

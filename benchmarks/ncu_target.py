@@ -3,7 +3,7 @@
     ncu --set full --clock-control none --import-source on -k regex:<kernel> -s 3 -c 1 -o gpurun_out/<name> \
         python benchmarks/ncu_target.py <what> <shape-name>
 
-what: fwd | fwd_stats | fwd_infer | dgrad | wgrad | bn_reduce | bn_apply | bn_bwd_apply | block_grad | stem_bwd_reduce | stem_bwd_apply | dwconv
+what: fwd | fwd_stats | fwd_infer | dgrad | wgrad | bn_reduce | bn_apply | bn_bwd_apply | block_grad | dwconv
 shape-name: one of gpu_check.BIG_SHAPES (e.g. s4_3x3_512)
 """
 import os
@@ -63,21 +63,6 @@ elif what == "block_grad":
     s0 = torch.zeros(cin, device="cuda"); s1 = torch.zeros(cin, device="cuda")
     dz = torch.empty(N, H, W, cin, device="cuda", dtype=torch.bfloat16)
     op = C.ConvDgrad(dy, w, dz, 1, 1, 1, 0, block_grad=(skip, mask, y3, s0, s1))
-elif what in ("stem_bwd_reduce", "stem_bwd_apply"):
-    Ho_ = 56
-    y0 = torch.randn(N, 2 * Ho_, 2 * Ho_, 64, device="cuda").to(torch.bfloat16)
-    sc = torch.ones(64, device="cuda"); sh = torch.zeros(64, device="cuda")
-    idx = torch.randint(0, 9, (N, Ho_, Ho_, 64), device="cuda", dtype=torch.uint8)
-    g1 = torch.randn(N, Ho_, Ho_, 64, device="cuda").to(torch.bfloat16); g2 = torch.randn_like(g1)
-    s0 = torch.zeros(64, device="cuda"); s1 = torch.zeros(64, device="cuda"); dy0 = torch.empty_like(y0)
-
-    class _Op:
-        def run(self):
-            if what == "stem_bwd_reduce":
-                e.stem_pool_bn_bwd(0, idx, g1, g2, y0, sc, sh, None, None, None, None, s0, s1)
-            else:
-                e.stem_pool_bn_bwd(1, idx, g1, g2, y0, sc, sh, sc, sh, sh, dy0, s0, s1)
-    op = _Op()
 elif what == "fwd_infer":
     # inference epilogue (kStats = 4): folded BatchNorm + ReLU + residual add in the GEMM epilogue (1x1 shapes take a residual)
     sc = torch.rand(cout, device="cuda") + 0.5; sh = torch.randn(cout, device="cuda") * 0.1

@@ -253,63 +253,6 @@ struct ConvPlan {
     keep.push_back(weight);
     keep.push_back(out);
   }
-  static float* f32(const at::Tensor& t, int64_t c, const char* name) {
-    TORCH_CHECK(t.is_cuda() && t.scalar_type() == at::kFloat && t.is_contiguous() && t.numel() >= c, name,
-                " must be a contiguous fp32 CUDA vector with >= Cout elements");
-    return t.data_ptr<float>();
-  }
-  static unsigned int* ctr(const at::Tensor& t) {
-    TORCH_CHECK(t.is_cuda() && t.scalar_type() == at::kInt && t.numel() >= 1, "counter must be an int32 CUDA tensor");
-    return reinterpret_cast<unsigned int*>(t.data_ptr<int>());
-  }
-  // kStats 1: the last CTA finalizes the BatchNorm whose statistics this GEMM accumulates (training mode)
-  void set_bn_finalize(at::Tensor counter, at::Tensor gamma, at::Tensor beta, at::Tensor rmean, at::Tensor rvar, at::Tensor mean,
-                       at::Tensor invstd, at::Tensor scale, at::Tensor shift, double count, double momentum, double eps) {
-    TORCH_CHECK(raw.stats == 1, "set_bn_finalize: the plan must have been created with statistics outputs");
-    const int64_t c = raw.p.cout;
-    auto& f = raw.p.fin;
-    f.counter = ctr(counter);
-    f.gamma = f32(gamma, c, "gamma");
-    f.beta = f32(beta, c, "beta");
-    f.running_mean = f32(rmean, c, "running_mean");
-    f.running_var = f32(rvar, c, "running_var");
-    f.mean = f32(mean, c, "mean");
-    f.invstd = f32(invstd, c, "invstd");
-    f.scale = f32(scale, c, "scale");
-    f.shift = f32(shift, c, "shift");
-    f.inv_count = (float)(1.0 / count);
-    f.unbias = count > 1 ? (float)(count / (count - 1.0)) : 1.f;
-    f.momentum = (float)momentum;
-    f.eps = (float)eps;
-    f.enable = 1;
-    for (auto& t : {counter, gamma, beta, rmean, rvar, mean, invstd, scale, shift}) keep.push_back(t);
-  }
-  // kStats 2 / 3: the last CTA turns sum(dz), sum(dz*y) into dgamma / dbeta and the apply coefficients A, B, C
-  void set_bn_bwd_coeffs(at::Tensor counter, at::Tensor gamma, at::Tensor mean, at::Tensor invstd, double count,
-                         at::Tensor dgamma, at::Tensor dbeta, at::Tensor cA, at::Tensor cB, at::Tensor cC) {
-    TORCH_CHECK(raw.stats == 2 || raw.stats == 3, "set_bn_bwd_coeffs: the plan must carry a fused BatchNorm-backward reduction");
-    const int64_t c = raw.p.cout;
-    auto& f = raw.p.bfin;
-    f.counter = ctr(counter);
-    f.gamma = f32(gamma, c, "gamma");
-    f.mean = f32(mean, c, "mean");
-    f.invstd = f32(invstd, c, "invstd");
-    f.dgamma = f32(dgamma, c, "dgamma");
-    f.dbeta = f32(dbeta, c, "dbeta");
-    f.cA = f32(cA, c, "cA");
-    f.cB = f32(cB, c, "cB");
-    f.cC = f32(cC, c, "cC");
-    f.inv_count = (float)(1.0 / count);
-    f.enable = 1;
-    for (auto& t : {counter, gamma, mean, invstd, dgamma, dbeta, cA, cB, cC}) keep.push_back(t);
-  }
-  // host-side switch (kernel parameters are captured by value at launch / graph-capture time): eval-mode forwards of a
-  // training engine must NOT update the running statistics
-  void enable_tail(bool on) {
-    if (raw.stats == 1 && raw.p.fin.counter != nullptr) raw.p.fin.enable = on ? 1 : 0;
-    if ((raw.stats == 2 || raw.stats == 3) && raw.p.bfin.counter != nullptr) raw.p.bfin.enable = on ? 1 : 0;
-  }
-  bool has_tail() const { return (raw.stats == 1 && raw.p.fin.counter != nullptr) || ((raw.stats == 2 || raw.stats == 3) && raw.p.bfin.counter != nullptr); }
   void run() {
     conv_plan_launch(raw, at::cuda::getCurrentCUDAStream());
     ++launches;
@@ -505,10 +448,6 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
            py::arg("relu_mask") = c10::nullopt, py::arg("ep_scale") = c10::nullopt, py::arg("ep_shift") = c10::nullopt,
            py::arg("ep_act") = 0)
       .def("run", &b200::ConvPlan::run)
-      .def("set_bn_finalize", &b200::ConvPlan::set_bn_finalize)
-      .def("set_bn_bwd_coeffs", &b200::ConvPlan::set_bn_bwd_coeffs)
-      .def("enable_tail", &b200::ConvPlan::enable_tail)
-      .def_property_readonly("has_tail", &b200::ConvPlan::has_tail)
       .def_readonly("launches", &b200::ConvPlan::launches)
       .def_property_readonly("grid", &b200::ConvPlan::grid)
       .def_property_readonly("block_n", &b200::ConvPlan::block_n)

@@ -615,52 +615,6 @@ conv_igemm_kernel(const __grid_constant__ TmapArray4 tmA, const __grid_constant_
         }
       }
     }
-    // ---- last-CTA tail: every CTA's sums are in L2 once its statistics threads have fenced and taken a ticket; the CTA
-    // that takes the last ticket turns the sums into the per-channel coefficients the NEXT kernel needs (and zeroes them),
-    // so no tiny dependent kernel sits between this GEMM and its consumer.
-    const bool want_tail = (kStats == 1) ? (p.fin.enable != 0) : (p.bfin.enable != 0);
-    if (want_tail) {
-      unsigned int* counter = (kStats == 1) ? p.fin.counter : p.bfin.counter;
-      int* s_last = reinterpret_cast<int*>(sStat);
-      __threadfence();
-      named_bar_sync(8, 128);
-      if (stid == 0) *s_last = (atomicAdd(counter, 1u) == gridDim.x - 1) ? 1 : 0;
-      named_bar_sync(8, 128);
-      if (*reinterpret_cast<volatile int*>(s_last) != 0) {
-        __threadfence();
-        for (int c = stid; c < p.cout; c += 128) {
-          const float s0 = __ldcg(p.stat_sum + c), s1 = __ldcg(p.stat_sqsum + c);
-          p.stat_sum[c] = 0.f;
-          p.stat_sqsum[c] = 0.f;
-          if (kStats == 1) {
-            const ConvParams::Fin& f = p.fin;
-            const float m = s0 * f.inv_count;
-            const float var = fmaxf(s1 * f.inv_count - m * m, 0.f);
-            f.running_mean[c] = (1.f - f.momentum) * f.running_mean[c] + f.momentum * m;
-            f.running_var[c] = (1.f - f.momentum) * f.running_var[c] + f.momentum * var * f.unbias;
-            const float is = rsqrtf(var + f.eps);
-            f.mean[c] = m;
-            f.invstd[c] = is;
-            const float sc = f.gamma[c] * is;
-            f.scale[c] = sc;
-            f.shift[c] = f.beta[c] - m * sc;
-          } else {
-            const ConvParams::BFin& f = p.bfin;
-            const float db = s0, dzy = s1;
-            const float m = f.mean[c], is = f.invstd[c];
-            const float dg = is * (dzy - m * db);
-            f.dgamma[c] = dg;
-            f.dbeta[c] = db;
-            const float A = f.gamma[c] * is;
-            const float B = -A * is * dg * f.inv_count;
-            f.cA[c] = A;
-            f.cB[c] = B;
-            f.cC[c] = -A * db * f.inv_count - B * m;
-          }
-        }
-        if (stid == 0) *counter = 0u;
-      }
-    }
   }
 
   tc_fence_before();

@@ -44,35 +44,6 @@ struct ConvParams {
   const float* ep_scale;
   const float* ep_shift;
   int ep_act;
-  // Last-CTA tails (replace the ~100 tiny dependent launches per step between the big kernels):
-  // kStats 1: BatchNorm finalize (batch statistics -> mean / invstd / scale / shift, running statistics update, sums zeroed)
-  struct Fin {
-    unsigned int* counter;  // zero between launches; the CTA that brings it to gridDim.x finalizes and resets it
-    const float* gamma;
-    const float* beta;
-    float* running_mean;
-    float* running_var;
-    float* mean;
-    float* invstd;
-    float* scale;
-    float* shift;
-    float inv_count, unbias, momentum, eps;
-    int enable;
-  } fin;
-  // kStats 2 / 3: BatchNorm-backward coefficients (dgamma, dbeta, dy = A*dz + B*y + C) from the sums this GEMM accumulated
-  struct BFin {
-    unsigned int* counter;
-    const float* gamma;
-    const float* mean;
-    const float* invstd;
-    float* dgamma;
-    float* dbeta;
-    float* cA;
-    float* cB;
-    float* cC;
-    float inv_count;
-    int enable;
-  } bfin;
 };
 
 // Weight-gradient GEMM:  dW[tap][co][ci] += sum_px dY[px, co] * X_tap[px, ci]

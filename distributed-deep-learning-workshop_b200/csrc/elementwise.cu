@@ -83,68 +83,16 @@ void bn_finalize(float* sum, float* sqsum, double count, const float* gamma, con
                                                       shift, C, training ? 1 : 0);
 }
 
-// In-kernel versions of bn_finalize_kernel / bn_bwd_coeffs_kernel for 8 consecutive channels (same expressions).
-__device__ __forceinline__ void bn_fwd_coeffs8(const BnFwdFuse& f, int c0, bool writer, float (&sc)[8], float (&sh)[8]) {
-  float su[8], sq[8], ga[8], be[8];
-  ldf8(f.sum + c0, su);
-  ldf8(f.sqsum + c0, sq);
-  ldf8(f.gamma + c0, ga);
-  ldf8(f.beta + c0, be);
-#pragma unroll
-  for (int k = 0; k < 8; ++k) {
-    const float m = su[k] * f.inv_count;
-    const float var = fmaxf(sq[k] * f.inv_count - m * m, 0.f);
-    const float is = rsqrtf(var + f.eps);
-    sc[k] = ga[k] * is;
-    sh[k] = be[k] - m * sc[k];
-    if (writer) {
-      const int c = c0 + k;
-      f.running_mean[c] = (1.f - f.momentum) * f.running_mean[c] + f.momentum * m;
-      f.running_var[c] = (1.f - f.momentum) * f.running_var[c] + f.momentum * var * f.unbias;
-      f.mean[c] = m;
-      f.invstd[c] = is;
-      f.scale[c] = sc[k];
-      f.shift[c] = sh[k];
-    }
-  }
-}
-__device__ __forceinline__ void bn_bwd_coeffs8(const BnBwdFuse& f, int c0, bool writer, float (&A)[8], float (&B)[8],
-                                               float (&Cc)[8]) {
-  float sz[8], szy[8], ga[8], me[8], is[8];
-  ldf8(f.sum_dz + c0, sz);
-  ldf8(f.sum_dzy + c0, szy);
-  ldf8(f.gamma + c0, ga);
-  ldf8(f.mean + c0, me);
-  ldf8(f.invstd + c0, is);
-#pragma unroll
-  for (int k = 0; k < 8; ++k) {
-    const float db = sz[k];
-    const float dg = is[k] * (szy[k] - me[k] * db);
-    A[k] = ga[k] * is[k];
-    B[k] = -A[k] * is[k] * dg * f.inv_count;
-    Cc[k] = -A[k] * db * f.inv_count - B[k] * me[k];
-    if (writer) {
-      f.dgamma[c0 + k] = dg;
-      f.dbeta[c0 + k] = db;
-    }
-  }
-}
-
 // ------------------------------------------------------------------------------------------------ BN apply
 // out = [relu]( y*scale + shift  [+ res | + res*res_scale + res_shift] )
 // Column-resident: a thread owns one 8-channel column vector and walks down the rows, so the per-channel
 // parameters are loaded into registers once instead of once per element (L1 traffic was 5x the payload).
-// U: rows per loop iteration.  All loads of the U rows are issued before the first is consumed: with one row per iteration a
-// thread has one or two 16-byte loads in flight and the kernel sits at ~64 % of the measured copy bandwidth (ncu: bn_bwd_apply
-// 4.2 of 6.57 TB/s at 34 % occupancy - too few bytes in flight for HBM3e's latency); the per-element arithmetic and its order
-// are unchanged, so every U produces bit-identical results.
-template <bool RELU, int RES, bool FUSED = false, int U = 1>  // RES: 0 none, 1 identity residual, 2 residual with its own BN
-__global__ void __launch_bounds__(256, U > 1 ? 3 : 1)
+template <bool RELU, int RES>  // RES: 0 none, 1 identity residual, 2 residual with its own BN
+__global__ void __launch_bounds__(256, 1)
 bn_apply_kernel(const __nv_bfloat16* __restrict__ y, const float* __restrict__ scale,
                 const float* __restrict__ shift, const __nv_bfloat16* __restrict__ res,
                 const float* __restrict__ res_scale, const float* __restrict__ res_shift,
-                __nv_bfloat16* __restrict__ out, uint8_t* __restrict__ mask, int64_t M, int C,
-                const BnFwdFuse fz = BnFwdFuse(), const BnFwdFuse rz = BnFwdFuse()) {
+                __nv_bfloat16* __restrict__ out, uint8_t* __restrict__ mask, int64_t M, int C) {
   const int cvec = C / 8;
   const int lanes = cvec < (int)blockDim.x ? cvec : blockDim.x;
   const int rpb = blockDim.x / lanes;
@@ -153,41 +101,25 @@ bn_apply_kernel(const __nv_bfloat16* __restrict__ y, const float* __restrict__ s
   if (ry >= rpb) return;
   for (int cv = cx; cv < cvec; cv += lanes) {
     float sc[8], sh[8], rs[8], rh[8];
-    if (FUSED) {
-      const bool writer = blockIdx.x == 0 && ry == 0;  // one thread per 8-channel column writes the saved statistics
-      bn_fwd_coeffs8(fz, cv * 8, writer, sc, sh);
-      if (RES == 2) bn_fwd_coeffs8(rz, cv * 8, writer, rs, rh);
-    } else {
-      ldf8(scale + cv * 8, sc);
-      ldf8(shift + cv * 8, sh);
-      if (RES == 2) {
-        ldf8(res_scale + cv * 8, rs);
-        ldf8(res_shift + cv * 8, rh);
-      }
+    ldf8(scale + cv * 8, sc);
+    ldf8(shift + cv * 8, sh);
+    if (RES == 2) {
+      ldf8(res_scale + cv * 8, rs);
+      ldf8(res_shift + cv * 8, rh);
     }
     const int64_t rstep = (int64_t)gridDim.x * rpb;
-    for (int64_t r0 = (int64_t)blockIdx.x * rpb + ry; r0 < M; r0 += rstep * U) {
-      bf16x8 yraw[U], rraw[U];
-#pragma unroll
-      for (int u = 0; u < U; ++u) {
-        const int64_t r = r0 + u * rstep;
-        if (r < M) {
-          yraw[u] = ld8(y + r * C + cv * 8);
-          if (RES >= 1) rraw[u] = ld8(res + r * C + cv * 8);
-        }
-      }
-#pragma unroll
-      for (int u = 0; u < U; ++u) {
-      const int64_t r = r0 + u * rstep;
-      if (r >= M) break;
+    for (int64_t r = (int64_t)blockIdx.x * rpb + ry; r < M; r += rstep) {
       const int64_t off = r * C + cv * 8;
+      const bf16x8 yraw = ld8(y + off);
+      bf16x8 rraw;
+      if (RES >= 1) rraw = ld8(res + off);
       float f[8];
-      unpack8(yraw[u], f);
+      unpack8(yraw, f);
 #pragma unroll
       for (int k = 0; k < 8; ++k) f[k] = fmaf(f[k], sc[k], sh[k]);
       if (RES >= 1) {
         float q[8];
-        unpack8(rraw[u], q);
+        unpack8(rraw, q);
         if (RES == 2) {
 #pragma unroll
           for (int k = 0; k < 8; ++k) q[k] = fmaf(q[k], rs[k], rh[k]);
@@ -206,18 +138,9 @@ bn_apply_kernel(const __nv_bfloat16* __restrict__ y, const float* __restrict__ s
         for (int k = 0; k < 8; ++k) f[k] = fmaxf(f[k], 0.f);
       }
       st8(out + off, pack8(f));
-      }
     }
   }
 }
-
-// rows per loop iteration of the BatchNorm apply / backward-apply kernels (1, 2 or 4); see bn_apply_kernel
-static int g_bn_rows_unroll = 1;
-// 3 = per-kernel choice from the measured table (profiles/r2_bn_unroll_check.txt): 4 rows for the forward apply without /
-// with an identity residual and for the mask-free backward apply, 2 rows for the backward apply that recomputes the ReLU mask,
-// 1 row for the apply with a second BatchNorm on the residual (more rows spill there)
-void set_bn_rows_unroll(int u) { g_bn_rows_unroll = (u == 2 || u == 3 || u == 4) ? u : 1; }
-int get_bn_rows_unroll() { return g_bn_rows_unroll; }
 
 static inline int rows_grid(int64_t M, int C, int threads) {
   const int cvec = C / 8;
@@ -239,40 +162,13 @@ void bn_apply(const void* y, const float* scale, const float* shift, const void*
   auto O = (__nv_bfloat16*)out;
   auto MK = (uint8_t*)mask;
   const int rmode = res == nullptr ? 0 : (res_scale == nullptr ? 1 : 2);
-#define LAUNCH(RL, RM)                                                                                               \
-  do {                                                                                                               \
-    if (g_bn_rows_unroll == 4 || (g_bn_rows_unroll == 3 && RM != 2))                                                 \
-      bn_apply_kernel<RL, RM, false, 4><<<blocks, threads, 0, s>>>(Y, scale, shift, R, res_scale, res_shift, O, MK, M, C); \
-    else if (g_bn_rows_unroll == 2)                                                                                  \
-      bn_apply_kernel<RL, RM, false, 2><<<blocks, threads, 0, s>>>(Y, scale, shift, R, res_scale, res_shift, O, MK, M, C); \
-    else                                                                                                             \
-      bn_apply_kernel<RL, RM><<<blocks, threads, 0, s>>>(Y, scale, shift, R, res_scale, res_shift, O, MK, M, C);     \
-  } while (0)
-  if (relu) {
-    if (rmode == 0) LAUNCH(true, 0); else if (rmode == 1) LAUNCH(true, 1); else LAUNCH(true, 2);
-  } else {
-    if (rmode == 0) LAUNCH(false, 0); else if (rmode == 1) LAUNCH(false, 1); else LAUNCH(false, 2);
-  }
-#undef LAUNCH
-}
-
-void bn_apply_fused(const void* y, const BnFwdFuse& f, const void* res, const BnFwdFuse* res_f, void* out, void* mask,
-                    int64_t M, int C, bool relu, cudaStream_t s) {
-  const int threads = 256;
-  const int blocks = rows_grid(M, C, threads);
-  auto Y = (const __nv_bfloat16*)y;
-  auto R = (const __nv_bfloat16*)res;
-  auto O = (__nv_bfloat16*)out;
-  auto MK = (uint8_t*)mask;
-  const int rmode = res == nullptr ? 0 : (res_f == nullptr ? 1 : 2);
-  const BnFwdFuse rz = res_f != nullptr ? *res_f : BnFwdFuse();
-#define LAUNCH(RL, RM) bn_apply_kernel<RL, RM, true><<<blocks, threads, 0, s>>>(Y, nullptr, nullptr, R, nullptr, nullptr, O, MK, M, C, f, rz)
-  if (relu) {
-    if (rmode == 0) LAUNCH(true, 0); else if (rmode == 1) LAUNCH(true, 1); else LAUNCH(true, 2);
-  } else {
-    if (rmode == 0) LAUNCH(false, 0); else if (rmode == 1) LAUNCH(false, 1); else LAUNCH(false, 2);
-  }
-#undef LAUNCH
+  const auto kernel = relu ? (rmode == 0   ? bn_apply_kernel<true, 0>
+                              : rmode == 1 ? bn_apply_kernel<true, 1>
+                                           : bn_apply_kernel<true, 2>)
+                           : (rmode == 0   ? bn_apply_kernel<false, 0>
+                              : rmode == 1 ? bn_apply_kernel<false, 1>
+                                           : bn_apply_kernel<false, 2>);
+  kernel<<<blocks, threads, 0, s>>>(Y, scale, shift, R, res_scale, res_shift, O, MK, M, C);
 }
 
 // ------------------------------------------------------------------------------------------------ channel stats
@@ -437,13 +333,12 @@ void bn_bwd_coeffs(float* sum_dz, float* sum_dzy, const float* gamma, const floa
 
 // dy = A*dz + B*y + Cc  with dz either read as-is (MASK=false: stored dz / BN without ReLU) or recomputed as
 // g * (y*scale + shift > 0) (MASK=true).  Column-resident like bn_apply_kernel.
-template <bool MASK, bool FUSED = false, int U = 1>   // U: rows per loop iteration (see bn_apply_kernel)
-__global__ void __launch_bounds__(256, U > 1 ? 3 : 1)
+template <bool MASK>
+__global__ void __launch_bounds__(256, 1)
 bn_bwd_apply_kernel(const __nv_bfloat16* __restrict__ g, const __nv_bfloat16* __restrict__ y,
                     const float* __restrict__ scale, const float* __restrict__ shift,
                     const float* __restrict__ cA, const float* __restrict__ cB,
-                    const float* __restrict__ cC, __nv_bfloat16* __restrict__ dy, int64_t M, int C,
-                    const BnBwdFuse fz = BnBwdFuse()) {
+                    const float* __restrict__ cC, __nv_bfloat16* __restrict__ dy, int64_t M, int C) {
   const int cvec = C / 8;
   const int lanes = cvec < (int)blockDim.x ? cvec : blockDim.x;
   const int rpb = blockDim.x / lanes;
@@ -452,44 +347,28 @@ bn_bwd_apply_kernel(const __nv_bfloat16* __restrict__ g, const __nv_bfloat16* __
   if (ry >= rpb) return;
   for (int cv = cx; cv < cvec; cv += lanes) {
     float A[8], B[8], Cc[8], sc[8], sh[8];
-    if (FUSED) {
-      bn_bwd_coeffs8(fz, cv * 8, blockIdx.x == 0 && ry == 0, A, B, Cc);
-    } else {
-      ldf8(cA + cv * 8, A);
-      ldf8(cB + cv * 8, B);
-      ldf8(cC + cv * 8, Cc);
-    }
+    ldf8(cA + cv * 8, A);
+    ldf8(cB + cv * 8, B);
+    ldf8(cC + cv * 8, Cc);
     if (MASK) {
       ldf8(scale + cv * 8, sc);
       ldf8(shift + cv * 8, sh);
     }
     const int64_t rstep = (int64_t)gridDim.x * rpb;
-    for (int64_t r0 = (int64_t)blockIdx.x * rpb + ry; r0 < M; r0 += rstep * U) {
-      bf16x8 graw[U], yraw[U];
+    for (int64_t r = (int64_t)blockIdx.x * rpb + ry; r < M; r += rstep) {
+      const int64_t off = r * C + cv * 8;
+      const bf16x8 graw = ld8(g + off);
+      const bf16x8 yraw = ld8(y + off);
+      float gg[8], yy[8];
+      unpack8(graw, gg);
+      unpack8(yraw, yy);
+      if (MASK) {
 #pragma unroll
-      for (int u = 0; u < U; ++u) {
-        const int64_t r = r0 + u * rstep;
-        if (r < M) {
-          graw[u] = ld8(g + r * C + cv * 8);
-          yraw[u] = ld8(y + r * C + cv * 8);
-        }
+        for (int k = 0; k < 8; ++k) gg[k] = fmaf(yy[k], sc[k], sh[k]) > 0.f ? gg[k] : 0.f;
       }
 #pragma unroll
-      for (int u = 0; u < U; ++u) {
-        const int64_t r = r0 + u * rstep;
-        if (r >= M) break;
-        const int64_t off = r * C + cv * 8;
-        float gg[8], yy[8];
-        unpack8(graw[u], gg);
-        unpack8(yraw[u], yy);
-        if (MASK) {
-#pragma unroll
-          for (int k = 0; k < 8; ++k) gg[k] = fmaf(yy[k], sc[k], sh[k]) > 0.f ? gg[k] : 0.f;
-        }
-#pragma unroll
-        for (int k = 0; k < 8; ++k) gg[k] = fmaf(A[k], gg[k], fmaf(B[k], yy[k], Cc[k]));
-        st8(dy + off, pack8(gg));
-      }
+      for (int k = 0; k < 8; ++k) gg[k] = fmaf(A[k], gg[k], fmaf(B[k], yy[k], Cc[k]));
+      st8(dy + off, pack8(gg));
     }
   }
 }
@@ -497,35 +376,9 @@ void bn_bwd_apply(const void* g, const void* y, const float* scale, const float*
                   const float* cB, const float* cC, void* dy, int64_t M, int C, cudaStream_t s) {
   const int threads = 256;
   const int blocks = rows_grid(M, C, threads);
-  auto G = (const __nv_bfloat16*)g;
-  auto Y = (const __nv_bfloat16*)y;
-  auto D = (__nv_bfloat16*)dy;
-#define LAUNCH_BWD(MK)                                                                                         \
-  do {                                                                                                         \
-    if (g_bn_rows_unroll == 4 || (g_bn_rows_unroll == 3 && !MK))                                               \
-      bn_bwd_apply_kernel<MK, false, 4><<<blocks, threads, 0, s>>>(G, Y, scale, shift, cA, cB, cC, D, M, C);    \
-    else if (g_bn_rows_unroll == 2 || (g_bn_rows_unroll == 3 && MK))                                           \
-      bn_bwd_apply_kernel<MK, false, 2><<<blocks, threads, 0, s>>>(G, Y, scale, shift, cA, cB, cC, D, M, C);    \
-    else                                                                                                       \
-      bn_bwd_apply_kernel<MK><<<blocks, threads, 0, s>>>(G, Y, scale, shift, cA, cB, cC, D, M, C);             \
-  } while (0)
-  if (scale != nullptr)
-    LAUNCH_BWD(true);
-  else
-    LAUNCH_BWD(false);
-#undef LAUNCH_BWD
-}
-
-void bn_bwd_apply_fused(const void* g, const void* y, const float* scale, const float* shift, const BnBwdFuse& f, void* dy,
-                        int64_t M, int C, cudaStream_t s) {
-  const int threads = 256;
-  const int blocks = rows_grid(M, C, threads);
-  if (scale != nullptr)
-    bn_bwd_apply_kernel<true, true><<<blocks, threads, 0, s>>>((const __nv_bfloat16*)g, (const __nv_bfloat16*)y, scale,
-                                                               shift, nullptr, nullptr, nullptr, (__nv_bfloat16*)dy, M, C, f);
-  else
-    bn_bwd_apply_kernel<false, true><<<blocks, threads, 0, s>>>((const __nv_bfloat16*)g, (const __nv_bfloat16*)y, scale,
-                                                                shift, nullptr, nullptr, nullptr, (__nv_bfloat16*)dy, M, C, f);
+  const auto kernel = scale != nullptr ? bn_bwd_apply_kernel<true> : bn_bwd_apply_kernel<false>;
+  kernel<<<blocks, threads, 0, s>>>((const __nv_bfloat16*)g, (const __nv_bfloat16*)y, scale, shift, cA, cB, cC,
+                                    (__nv_bfloat16*)dy, M, C);
 }
 
 // ------------------------------------------------------------------------------------------------ max pool 3x3 s2 p1
@@ -826,24 +679,6 @@ void softmax_ce(const float* logits, const int64_t* labels, float* dlogits, floa
   const int threads = 128;
   const int blocks = (B * 32 + threads - 1) / threads;
   softmax_ce_kernel<<<blocks, threads, 0, s>>>(logits, labels, dlogits, loss_rows, stats, B, K, grad_scale);
-}
-
-// ------------------------------------------------------------------------------------------------ preprocess
-// uint8 NHWC [N,H,W,3] -> bf16 NHWC [N,H,W,Cpad] with x/127.5 - 1 (MobileNet/Keras "preprocess_input" rule, C13);
-// padded channels are zero so the stem can run as a tensor-core GEMM.
-__global__ void preprocess_u8_kernel(const uint8_t* __restrict__ x, __nv_bfloat16* __restrict__ out, int64_t npix,
-                                     int cpad, float mul, float add) {
-  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < npix; i += (int64_t)gridDim.x * blockDim.x) {
-    const uint8_t* p = x + i * 3;
-    __nv_bfloat16* o = out + i * cpad;
-    o[0] = __float2bfloat16(fmaf((float)p[0], mul, add));
-    o[1] = __float2bfloat16(fmaf((float)p[1], mul, add));
-    o[2] = __float2bfloat16(fmaf((float)p[2], mul, add));
-    for (int c = 3; c < cpad; ++c) o[c] = __float2bfloat16(0.f);
-  }
-}
-void preprocess_u8(const uint8_t* x, void* out, int64_t npix, int cpad, float mul, float add, cudaStream_t s) {
-  preprocess_u8_kernel<<<grid_for(npix, 256), 256, 0, s>>>(x, (__nv_bfloat16*)out, npix, cpad, mul, add);
 }
 
 // Bilinear resize (half-pixel centres, like tf.image.resize) of one uint8 image batch to [N, OH, OW, 3] uint8 (HWC).

@@ -1,12 +1,9 @@
-// Classifier-head and stem-tail kernels (SURVEY.md K11, K14, K15): the bandwidth-bound glue around the two GEMM-shaped
+// Classifier-head and stem-weight kernels (SURVEY.md K11, K14, K15): the bandwidth-bound glue around the two GEMM-shaped
 // ends of the network.  The FC layer itself runs on the tcgen05 implicit-GEMM kernels (a 1x1 "convolution" over a 1x1
 // image, csrc/conv_igemm.cuh / conv_wgrad.cu); what lives here is everything the reference's Dense + softmax head
-// (P1/02:175) and MaxPool backward need besides the GEMMs:
+// (P1/02:175) needs besides the GEMMs:
 //   * softmax_ce_head: bf16 logits + fp32 bias -> loss, accuracy, bf16 dlogits (padded columns zero) in one pass;
 //   * fc_bias_grad: column sums of dlogits;
-//   * stem_pool_bn_bwd: 3x3/2 max-pool backward (argmax scatter) fused with the stem BatchNorm+ReLU backward - the
-//     112x112x64 pooled-gradient tensor is never written: pass 0 reduces sum(dz), sum(dz*y), pass 1 writes dy;
-//     both rebuild the pooled gradient of a 16x16-pixel tile in shared memory (conflict-free colour-class scatter);
 //   * pack_stem_weight: fp32 [49, 64, 3] master -> bf16 [64, 192] GEMM operand.
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
@@ -15,29 +12,6 @@
 #include "ops_api.h"
 
 namespace b200 {
-
-namespace {
-
-struct alignas(16) bf8 {
-  __nv_bfloat162 v[4];
-};
-__device__ __forceinline__ void unpack8h(const bf8& p, float (&f)[8]) {
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    float2 t = __bfloat1622float2(p.v[i]);
-    f[2 * i] = t.x;
-    f[2 * i + 1] = t.y;
-  }
-}
-__device__ __forceinline__ bf8 pack8h(const float (&f)[8]) {
-  bf8 p;
-#pragma unroll
-  for (int i = 0; i < 4; ++i) p.v[i] = __floats2bfloat162_rn(f[2 * i], f[2 * i + 1]);
-  return p;
-}
-__device__ __forceinline__ float bf16_round(float x) { return __bfloat162float(__float2bfloat16(x)); }
-
-}  // namespace
 
 // ------------------------------------------------------------------------------------------------ softmax CE head
 // One warp per row.  logit[k] = bf16 logits16[row, k] + bias[k] for k < K (row pitch ld >= K, padded columns ignored).
@@ -125,188 +99,6 @@ __global__ void pack_stem_weight_kernel(const float* __restrict__ w, __nv_bfloat
 }
 void pack_stem_weight(const float* w, void* out, cudaStream_t s) {
   pack_stem_weight_kernel<<<(64 * 192 + 255) / 256, 256, 0, s>>>(w, (__nv_bfloat16*)out);
-}
-
-// ------------------------------------------------------------------------------------------------ stem tail backward
-// Backward of  p = maxpool3x3/2( relu( y*scale + shift ) )  for the 64-channel stem, without materialising the pooled
-// gradient on the 2Ho x 2Wo grid:
-//   da[h, w]  = sum over the <= 4 windows containing (h, w) whose saved argmax is this position of (g1 + g2)[ho, wo]
-//   dz        = da * [y*scale + shift > 0]
-//   PASS 0:   sum_dz += dz, sum_dzy += dz * y          (per channel; one flush of atomics per CTA)
-//   PASS 1:   dy = cA*dz + cB*y + cC
-// v1 of this kernel GATHERED per input pixel (compare the saved argmax of up to four windows, per channel) and was
-// instruction-bound: ncu 327 M warp instructions per pass, DRAM 15 % (profiles/r2_ncu_stem_bwd_*_v1.txt) - slower than the
-// three-kernel path it replaced.  v2 SCATTERS: every window contributes its gradient to exactly ONE pixel (its argmax), so
-// a CTA builds the da tile of 16x16 pixels x 64 channels in shared memory (fp32, 64 KB) by read-modify-write:
-//   * a warp handles (window, 32-channel half); lane = channel, so the smem bank is the lane whatever pixel is hit;
-//   * windows are processed in four colour classes (row parity x column parity): windows of one class have disjoint 3x3
-//     footprints, so plain (non-atomic) updates are race-free inside a class; __syncthreads between classes
-//     (shared-memory fp32 atomicAdd is a CAS spin loop on sm_100a - ATOMS.CAST.SPIN - and would dominate);
-//   * then the pixel phase reads da from smem, y from global, and reduces / applies.
-constexpr int kPoolTile = 8;
-constexpr int kPoolWin = kPoolTile + 1;
-constexpr int kStemDaBytes = 16 * 16 * 64 * 4;
-
-template <int PASS>
-__global__ void __launch_bounds__(256, 3)
-stem_pool_bn_bwd_kernel(const uint8_t* __restrict__ idx, const __nv_bfloat16* __restrict__ g1,
-                        const __nv_bfloat16* __restrict__ g2, const __nv_bfloat16* __restrict__ y,
-                        const float* __restrict__ scale, const float* __restrict__ shift,
-                        const float* __restrict__ cA, const float* __restrict__ cB, const float* __restrict__ cC,
-                        __nv_bfloat16* __restrict__ dy, float* __restrict__ sum_dz, float* __restrict__ sum_dzy, int N,
-                        int Ho, int Wo) {
-  constexpr int C = 64;
-  extern __shared__ __align__(16) float da[];  // [256 pixels][64 channels]
-  __shared__ float red[2][8][C];
-  const int H = 2 * Ho, W = 2 * Wo;
-  const int tiles_h = Ho / kPoolTile, tiles_w = Wo / kPoolTile;
-  const int num_tiles = N * tiles_h * tiles_w;
-  const int t = threadIdx.x;
-  const int warp = t >> 5, lane = t & 31;
-  const int cv = t & 7;
-  const int pl = t >> 3;  // 0..31: pixel lane; pixels p = pl + 32*i
-  float sc[8], sh[8], A[8], B[8], Cc[8], t0[8], t1[8];
-#pragma unroll
-  for (int k = 0; k < 8; ++k) {
-    sc[k] = scale[cv * 8 + k];
-    sh[k] = shift[cv * 8 + k];
-    t0[k] = t1[k] = 0.f;
-    if (PASS == 1) {
-      A[k] = cA[cv * 8 + k];
-      B[k] = cB[cv * 8 + k];
-      Cc[k] = cC[cv * 8 + k];
-    }
-  }
-  for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-    const int tb = tile % tiles_w;
-    const int rest = tile / tiles_w;
-    const int ta = rest % tiles_h;
-    const int n = rest / tiles_h;
-    const int a0 = ta * kPoolTile, b0 = tb * kPoolTile;
-    __syncthreads();  // the previous tile's pixel phase is done with da
-    for (int i = t; i < 16 * 16 * C / 4; i += 256) reinterpret_cast<float4*>(da)[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-    __syncthreads();
-#pragma unroll 1
-    for (int cls = 0; cls < 4; ++cls) {
-      const int ci = cls >> 1, cj = cls & 1;
-      const int nwj = (kPoolWin - 1 - cj) / 2 + 1;
-      const int items = ((kPoolWin - 1 - ci) / 2 + 1) * nwj * 2;
-      // A warp owns at most kMaxIt = 7 (window, half) items of a class (<= 25 windows x 2 halves over 8 warps): ALL their
-      // global loads are issued before the first read-modify-write, so ~7 x 5 bytes per lane are in flight instead of one
-      // item's (v2a: ncu 58 % long-scoreboard stalls in this loop, 16 % DRAM throughput).
-      constexpr int kMaxIt = 7;
-      int a_[kMaxIt];   // bits 0-7 argmax position, 8-15 wi, 16-23 wj, bit 30 = item present
-      float g_[kMaxIt];
-      const int ch = (warp & 1) * 32 + lane;  // it = warp + 8q: the channel half of all of a warp's items is warp & 1
-#pragma unroll
-      for (int q = 0; q < kMaxIt; ++q) {
-        const int it = warp + 8 * q;
-        a_[q] = 0;
-        g_[q] = 0.f;
-        if (it < items) {
-          const int w = it >> 1;
-          const int wi = ci + 2 * (w / nwj), wj = cj + 2 * (w % nwj);
-          const int ho = a0 + wi, wo = b0 + wj;
-          if (ho < Ho && wo < Wo) {  // warp-uniform
-            const int64_t o = ((((int64_t)n * Ho + ho) * Wo + wo) * C) + ch;
-            a_[q] = static_cast<int>(idx[o]) | (wi << 8) | (wj << 16) | (1 << 30);
-            g_[q] = __bfloat162float(g1[o]);
-            if (g2 != nullptr) g_[q] += __bfloat162float(g2[o]);
-          }
-        }
-      }
-#pragma unroll
-      for (int q = 0; q < kMaxIt; ++q) {
-        if (a_[q] != 0) {
-          const int a = a_[q] & 0xFF, wi = (a_[q] >> 8) & 0xFF, wj = (a_[q] >> 16) & 0xFF;
-          const int r = (a * 11) >> 5;  // a / 3 for a in 0..8
-          const int row = 2 * wi - 1 + r, col = 2 * wj - 1 + (a - 3 * r);
-          if (static_cast<unsigned>(row) < 16u && static_cast<unsigned>(col) < 16u) da[(row * 16 + col) * C + ch] += g_[q];
-        }
-      }
-      __syncthreads();
-    }
-    const int pw = pl & 15;
-#pragma unroll 2
-    for (int i = 0; i < 8; ++i) {
-      const int ph = (pl >> 4) + 2 * i;
-      const int h = 2 * a0 + ph, w = 2 * b0 + pw;
-      const float4 d0 = *reinterpret_cast<const float4*>(&da[(ph * 16 + pw) * C + cv * 8]);
-      const float4 d1 = *reinterpret_cast<const float4*>(&da[(ph * 16 + pw) * C + cv * 8 + 4]);
-      const float acc[8] = {d0.x, d0.y, d0.z, d0.w, d1.x, d1.y, d1.z, d1.w};
-      const int64_t off = ((((int64_t)n * H + h) * W + w) * C) + cv * 8;
-      float yy[8];
-      unpack8h(*reinterpret_cast<const bf8*>(y + off), yy);
-      float dz[8];
-#pragma unroll
-      for (int k = 0; k < 8; ++k) {
-        // bf16 rounding of the pooled gradient: same values as the materialised path (maxpool_bwd -> bf16 tensor)
-        const float a = bf16_round(acc[k]);
-        dz[k] = fmaf(yy[k], sc[k], sh[k]) > 0.f ? a : 0.f;
-      }
-      if (PASS == 0) {
-#pragma unroll
-        for (int k = 0; k < 8; ++k) {
-          t0[k] += dz[k];
-          t1[k] = fmaf(dz[k], yy[k], t1[k]);
-        }
-      } else {
-        float o8[8];
-#pragma unroll
-        for (int k = 0; k < 8; ++k) o8[k] = fmaf(A[k], dz[k], fmaf(B[k], yy[k], Cc[k]));
-        *reinterpret_cast<bf8*>(dy + off) = pack8h(o8);
-      }
-    }
-  }
-  if (PASS == 0) {
-    // lanes with equal (lane & 7) own the same 8 channels: fold the 4 pixel lanes of a warp, then the 8 warps
-#pragma unroll
-    for (int k = 0; k < 8; ++k) {
-      t0[k] += __shfl_xor_sync(0xffffffffu, t0[k], 8);
-      t0[k] += __shfl_xor_sync(0xffffffffu, t0[k], 16);
-      t1[k] += __shfl_xor_sync(0xffffffffu, t1[k], 8);
-      t1[k] += __shfl_xor_sync(0xffffffffu, t1[k], 16);
-    }
-    __syncthreads();
-    if (lane < 8) {
-#pragma unroll
-      for (int k = 0; k < 8; ++k) {
-        red[0][warp][lane * 8 + k] = t0[k];
-        red[1][warp][lane * 8 + k] = t1[k];
-      }
-    }
-    __syncthreads();
-    if (t < 2 * C) {
-      const int which = t / C, c = t % C;
-      float a = 0.f;
-#pragma unroll
-      for (int wv = 0; wv < 8; ++wv) a += red[which][wv][c];
-      atomicAdd((which == 0 ? sum_dz : sum_dzy) + c, a);
-    }
-  }
-}
-
-// pass 0: reduce (sum_dz, sum_dzy accumulate);  pass 1: apply (dy written)
-void stem_pool_bn_bwd(int pass, const void* idx, const void* g1, const void* g2, const void* y, const float* scale,
-                      const float* shift, const float* cA, const float* cB, const float* cC, void* dy, float* sum_dz,
-                      float* sum_dzy, int N, int Ho, int Wo, cudaStream_t s) {
-  static bool attr_set = false;
-  if (!attr_set) {
-    cudaFuncSetAttribute(stem_pool_bn_bwd_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kStemDaBytes);
-    cudaFuncSetAttribute(stem_pool_bn_bwd_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kStemDaBytes);
-    attr_set = true;
-  }
-  const int tiles = N * (Ho / kPoolTile) * (Wo / kPoolTile);
-  int grid = 148 * 3;
-  if (grid > tiles) grid = tiles;
-  if (pass == 0)
-    stem_pool_bn_bwd_kernel<0><<<grid, 256, kStemDaBytes, s>>>((const uint8_t*)idx, (const __nv_bfloat16*)g1,
-                                                               (const __nv_bfloat16*)g2, (const __nv_bfloat16*)y, scale,
-                                                               shift, cA, cB, cC, (__nv_bfloat16*)dy, sum_dz, sum_dzy, N, Ho, Wo);
-  else
-    stem_pool_bn_bwd_kernel<1><<<grid, 256, kStemDaBytes, s>>>((const uint8_t*)idx, (const __nv_bfloat16*)g1,
-                                                               (const __nv_bfloat16*)g2, (const __nv_bfloat16*)y, scale,
-                                                               shift, cA, cB, cC, (__nv_bfloat16*)dy, sum_dz, sum_dzy, N, Ho, Wo);
 }
 
 }  // namespace b200

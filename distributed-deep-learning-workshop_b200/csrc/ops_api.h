@@ -5,41 +5,9 @@
 
 namespace b200 {
 
-// Optional in-kernel BatchNorm coefficient computation (replaces a separate bn_finalize / bn_bwd_coeffs launch on the
-// critical path).  sum == nullptr / sum_dz == nullptr selects the unfused behaviour (coefficients read from arrays).
-struct BnFwdFuse {
-  const float* sum;      // per-channel sum(y), sum(y^2) accumulated by the conv epilogue (zeroed once per step by the engine)
-  const float* sqsum;
-  const float* gamma;
-  const float* beta;
-  float* running_mean;   // updated by the first row-block
-  float* running_var;
-  float* mean;           // written by the first row-block for the backward pass
-  float* invstd;
-  float* scale;
-  float* shift;
-  float inv_count, unbias, momentum, eps;
-};
-struct BnBwdFuse {
-  const float* sum_dz;   // per-channel sum(dz), sum(dz*y) (zeroed once per step by the engine)
-  const float* sum_dzy;
-  const float* gamma;
-  const float* mean;
-  const float* invstd;
-  float* dgamma;         // written by the first row-block
-  float* dbeta;
-  float inv_count;
-};
-void bn_apply_fused(const void* y, const BnFwdFuse& f, const void* res, const BnFwdFuse* res_f, void* out, void* mask,
-                    int64_t M, int C, bool relu, cudaStream_t s);
-void bn_bwd_apply_fused(const void* g, const void* y, const float* scale, const float* shift, const BnBwdFuse& f, void* dy,
-                        int64_t M, int C, cudaStream_t s);
 void bn_finalize(float* sum, float* sqsum, double count, const float* gamma, const float* beta, float* running_mean,
                  float* running_var, float momentum, float eps, float* mean, float* invstd, float* scale,
                  float* shift, int C, bool training, cudaStream_t s);
-// rows per loop iteration of the BatchNorm apply / backward-apply kernels: 1 (default), 2 or 4 - bit-identical results
-void set_bn_rows_unroll(int u);
-int get_bn_rows_unroll();
 void bn_apply(const void* y, const float* scale, const float* shift, const void* res, const float* res_scale,
               const float* res_shift, void* out, void* mask, int64_t M, int C, bool relu, cudaStream_t s);
 void channel_stats(const void* y, float* sum, float* sqsum, int64_t M, int C, cudaStream_t s);
@@ -62,14 +30,10 @@ void softmax_ce_head(const void* logits16, int ld, const float* bias, const int6
                      void* dlogits16, float* loss_rows, float* stats, int B, int K, float grad_scale, cudaStream_t s);
 void fc_bias_grad(const void* dlogits16, int ld, float* dbias, int B, int K, cudaStream_t s);
 void pack_stem_weight(const float* w, void* out, cudaStream_t s);
-void stem_pool_bn_bwd(int pass, const void* idx, const void* g1, const void* g2, const void* y, const float* scale,
-                      const float* shift, const float* cA, const float* cB, const float* cC, void* dy, float* sum_dz,
-                      float* sum_dzy, int N, int Ho, int Wo, cudaStream_t s);
 void mbv2_stem(const uint8_t* x, const float* w, const float* scale, const float* shift, void* out, int N, int H, int W,
                int ldc, float mul, float add, cudaStream_t s);
 void dwconv3x3(const void* x, const float* w, const float* scale, const float* shift, void* out, int N, int H, int W, int C,
                int stride, int tile_w, cudaStream_t s);
-void preprocess_u8(const uint8_t* x, void* out, int64_t npix, int cpad, float mul, float add, cudaStream_t s);
 void resize_bilinear_u8(const uint8_t* x, uint8_t* out, int N, int H, int W, int OH, int OW, bool planar, cudaStream_t s);
 void weight_prep(const float* w, void* wf, void* wd, int taps, int cout, int cin, cudaStream_t s);
 void weight_prep_batched(const float* params, void* wd, const int64_t* table, int layers, int64_t total,

@@ -3,7 +3,6 @@
 #include <torch/extension.h>
 
 #include <cstdint>
-#include <vector>
 
 #include "ops_api.h"
 
@@ -97,73 +96,6 @@ void bn_bwd_apply(Tensor g, Tensor y, OptT scale, OptT shift, Tensor cA, Tensor 
   after();
 }
 
-// ---- fused variants: the BatchNorm coefficients are computed inside the consumer kernel (no bn_finalize / bn_bwd_coeffs
-// launch on the critical path); the caller zeroes the sum accumulators once per step.
-static b200::BnFwdFuse fwd_fuse(const Tensor& sum, const Tensor& sqsum, const Tensor& gamma, const Tensor& beta,
-                                const Tensor& rmean, const Tensor& rvar, const Tensor& mean, const Tensor& invstd,
-                                const Tensor& scale, const Tensor& shift, double count, double momentum, double eps, int C) {
-  for (const Tensor* t : {&sum, &sqsum, &gamma, &beta, &rmean, &rvar, &mean, &invstd, &scale, &shift}) {
-    TORCH_CHECK(t->is_cuda() && t->scalar_type() == at::kFloat && t->numel() == C && t->is_contiguous(),
-                "fused BN parameter must be a contiguous fp32 CUDA vector of C elements");
-    TORCH_CHECK(reinterpret_cast<uintptr_t>(t->data_ptr()) % 16 == 0, "fused BN parameter must be 16-byte aligned");
-  }
-  b200::BnFwdFuse f;
-  f.sum = sum.data_ptr<float>(); f.sqsum = sqsum.data_ptr<float>();
-  f.gamma = gamma.data_ptr<float>(); f.beta = beta.data_ptr<float>();
-  f.running_mean = rmean.data_ptr<float>(); f.running_var = rvar.data_ptr<float>();
-  f.mean = mean.data_ptr<float>(); f.invstd = invstd.data_ptr<float>();
-  f.scale = scale.data_ptr<float>(); f.shift = shift.data_ptr<float>();
-  f.inv_count = (float)(1.0 / count);
-  f.unbias = count > 1 ? (float)(count / (count - 1.0)) : 1.f;
-  f.momentum = (float)momentum;
-  f.eps = (float)eps;
-  return f;
-}
-
-// pack order (main BN and `res_pack`): sum, sqsum, gamma, beta, running_mean, running_var, mean, invstd, scale, shift
-void bn_apply_fused(Tensor y, std::vector<Tensor> pack, double count, double momentum, double eps, OptT res,
-                    c10::optional<std::vector<Tensor>> res_pack, Tensor out, bool relu, OptT mask) {
-  chk(y, at::kBFloat16, "y");
-  chk(out, at::kBFloat16, "out");
-  const int C = (int)y.size(-1);
-  const int64_t M = y.numel() / C;
-  TORCH_CHECK(C % 8 == 0 && out.numel() == y.numel() && pack.size() == 10);
-  if (res.has_value()) { chk(*res, at::kBFloat16, "res"); TORCH_CHECK(res->numel() == y.numel()); }
-  if (mask.has_value()) { chk(*mask, at::kByte, "mask"); TORCH_CHECK(mask->numel() * 8 == y.numel()); }
-  TORCH_CHECK(!res_pack.has_value() || res.has_value(), "res_pack needs res");
-  b200::BnFwdFuse f = fwd_fuse(pack[0], pack[1], pack[2], pack[3], pack[4], pack[5], pack[6], pack[7], pack[8], pack[9],
-                               count, momentum, eps, C);
-  b200::BnFwdFuse rf;
-  if (res_pack.has_value()) {
-    const auto& q = *res_pack;
-    TORCH_CHECK(q.size() == 10);
-    rf = fwd_fuse(q[0], q[1], q[2], q[3], q[4], q[5], q[6], q[7], q[8], q[9], count, momentum, eps, C);
-  }
-  b200::bn_apply_fused(y.data_ptr(), f, vp(res), res_pack.has_value() ? &rf : nullptr, out.data_ptr(),
-                       mask.has_value() ? mask->data_ptr() : nullptr, M, C, relu, cur());
-  after();
-}
-
-// dy = A*dz + B*y + C with A, B, C computed in the kernel from sum_dz, sum_dzy; dgamma / dbeta written by the kernel.
-void bn_bwd_apply_fused(Tensor g, Tensor y, OptT scale, OptT shift, Tensor sum_dz, Tensor sum_dzy, Tensor gamma,
-                        Tensor mean, Tensor invstd, double count, Tensor dgamma, Tensor dbeta, Tensor dy) {
-  chk(g, at::kBFloat16, "g");
-  chk(y, at::kBFloat16, "y");
-  chk(dy, at::kBFloat16, "dy");
-  const int C = (int)y.size(-1);
-  for (const Tensor* t : {&sum_dz, &sum_dzy, &gamma, &mean, &invstd, &dgamma, &dbeta}) {
-    TORCH_CHECK(t->is_cuda() && t->scalar_type() == at::kFloat && t->numel() == C && t->is_contiguous());
-    TORCH_CHECK(reinterpret_cast<uintptr_t>(t->data_ptr()) % 16 == 0, "fused BN parameter must be 16-byte aligned");
-  }
-  b200::BnBwdFuse f;
-  f.sum_dz = sum_dz.data_ptr<float>(); f.sum_dzy = sum_dzy.data_ptr<float>();
-  f.gamma = gamma.data_ptr<float>(); f.mean = mean.data_ptr<float>(); f.invstd = invstd.data_ptr<float>();
-  f.dgamma = dgamma.data_ptr<float>(); f.dbeta = dbeta.data_ptr<float>();
-  f.inv_count = (float)(1.0 / count);
-  b200::bn_bwd_apply_fused(g.data_ptr(), y.data_ptr(), fp(scale), fp(shift), f, dy.data_ptr(), y.numel() / C, C, cur());
-  after();
-}
-
 void maxpool_fwd(Tensor x, Tensor out, OptT idx) {
   chk(x, at::kBFloat16, "x");
   chk(out, at::kBFloat16, "out");
@@ -248,26 +180,6 @@ void pack_stem_weight(Tensor w, Tensor out) {
   b200::pack_stem_weight(w.data_ptr<float>(), out.data_ptr(), cur());
   after();
 }
-// max-pool 3x3/2 backward fused with the stem BN+ReLU backward; pass 0 = reduce, pass 1 = apply (see head_stem.cu)
-void stem_pool_bn_bwd(int64_t pass, Tensor idx, Tensor g1, OptT g2, Tensor y, Tensor scale, Tensor shift, OptT cA, OptT cB,
-                      OptT cC, OptT dy, Tensor sum_dz, Tensor sum_dzy) {
-  chk(idx, at::kByte, "idx");
-  chk(g1, at::kBFloat16, "g1");
-  chk(y, at::kBFloat16, "y");
-  chk(scale, at::kFloat, "scale");
-  chk(shift, at::kFloat, "shift");
-  TORCH_CHECK(y.dim() == 4 && y.size(3) == 64 && g1.dim() == 4 && g1.size(3) == 64, "stem tail: 64 channels, NHWC");
-  const int N = (int)g1.size(0), Ho = (int)g1.size(1), Wo = (int)g1.size(2);
-  TORCH_CHECK(y.size(0) == N && y.size(1) == 2 * Ho && y.size(2) == 2 * Wo && idx.numel() == g1.numel());
-  TORCH_CHECK(Ho % 8 == 0 && Wo % 8 == 0, "stem tail: pooled grid must tile by 8");
-  if (g2.has_value()) { chk(*g2, at::kBFloat16, "g2"); TORCH_CHECK(g2->numel() == g1.numel()); }
-  TORCH_CHECK(pass == 0 || (cA.has_value() && cB.has_value() && cC.has_value() && dy.has_value()));
-  if (dy.has_value()) { chk(*dy, at::kBFloat16, "dy"); TORCH_CHECK(dy->numel() == y.numel()); }
-  b200::stem_pool_bn_bwd((int)pass, idx.data_ptr(), g1.data_ptr(), vp(g2), y.data_ptr(), scale.data_ptr<float>(),
-                         shift.data_ptr<float>(), fp(cA), fp(cB), fp(cC), dy.has_value() ? dy->data_ptr() : nullptr,
-                         sum_dz.data_ptr<float>(), sum_dzy.data_ptr<float>(), N, Ho, Wo, cur());
-  after();
-}
 // cudaMemsetAsync on the current stream (a memset node under graph capture, not a kernel)
 void zero_(Tensor t) {
   TORCH_CHECK(t.is_cuda() && t.is_contiguous());
@@ -302,13 +214,6 @@ void dwconv3x3(Tensor x, Tensor w, Tensor scale, Tensor shift, Tensor out, int64
               out.size(2) == (W - 1) / stride + 1, "dwconv3x3 output shape");
   b200::dwconv3x3(x.data_ptr(), w.data_ptr<float>(), scale.data_ptr<float>(), shift.data_ptr<float>(), out.data_ptr(),
                   (int)x.size(0), H, W, C, (int)stride, (int)tile_w, cur());
-  after();
-}
-void preprocess_u8(Tensor x, Tensor out, double mul, double add) {
-  chk(x, at::kByte, "x");
-  chk(out, at::kBFloat16, "out");
-  TORCH_CHECK(x.size(-1) == 3);
-  b200::preprocess_u8(x.data_ptr<uint8_t>(), out.data_ptr(), x.numel() / 3, (int)out.size(-1), (float)mul, (float)add, cur());
   after();
 }
 // x: uint8 [N, H, W, 3] (planar = false) or [N, 3, H, W] (planar = true, the nvJPEG layout);  out: uint8 [N, OH, OW, 3]
@@ -380,10 +285,6 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
   m.def("bn_bwd_reduce", &bn_bwd_reduce);
   m.def("bn_bwd_coeffs", &bn_bwd_coeffs);
   m.def("bn_bwd_apply", &bn_bwd_apply);
-  m.def("bn_apply_fused", &bn_apply_fused, py::arg("y"), py::arg("pack"), py::arg("count"), py::arg("momentum"),
-        py::arg("eps"), py::arg("res") = c10::nullopt, py::arg("res_pack") = c10::nullopt, py::arg("out"),
-        py::arg("relu") = true, py::arg("mask") = c10::nullopt);
-  m.def("bn_bwd_apply_fused", &bn_bwd_apply_fused);
   m.def("maxpool_fwd", &maxpool_fwd);
   m.def("maxpool_bwd", &maxpool_bwd);
   m.def("bn_relu_maxpool_fwd", &bn_relu_maxpool_fwd);
@@ -395,16 +296,10 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
         py::arg("stats"), py::arg("grad_scale") = 1.0);
   m.def("fc_bias_grad", &fc_bias_grad);
   m.def("pack_stem_weight", &pack_stem_weight);
-  m.def("stem_pool_bn_bwd", &stem_pool_bn_bwd, py::arg("pass_"), py::arg("idx"), py::arg("g1"), py::arg("g2"), py::arg("y"),
-        py::arg("scale"), py::arg("shift"), py::arg("cA") = c10::nullopt, py::arg("cB") = c10::nullopt,
-        py::arg("cC") = c10::nullopt, py::arg("dy") = c10::nullopt, py::arg("sum_dz"), py::arg("sum_dzy"));
   m.def("zero_", &zero_);
-  m.def("set_bn_rows_unroll", [](int64_t u) { b200::set_bn_rows_unroll((int)u); });
-  m.def("get_bn_rows_unroll", []() { return (int64_t)b200::get_bn_rows_unroll(); });
   m.def("mbv2_stem", &mbv2_stem);
   m.def("dwconv3x3", &dwconv3x3, pybind11::arg("x"), pybind11::arg("w"), pybind11::arg("scale"), pybind11::arg("shift"),
         pybind11::arg("out"), pybind11::arg("stride"), pybind11::arg("tile_w") = 4);
-  m.def("preprocess_u8", &preprocess_u8);
   m.def("resize_bilinear_u8", &resize_bilinear_u8, py::arg("x"), py::arg("out"), py::arg("planar") = false);
   m.def("weight_prep", &weight_prep);
   m.def("weight_prep_batched", &weight_prep_batched);

@@ -85,45 +85,32 @@ class ResNet50Engine:
 
     def __init__(self, batch: int, num_classes: int = 1000, device: Optional[torch.device] = None,
                  image_size: int = 224, dropout: float = 0.0, bn_momentum: float = 0.1, bn_eps: float = 1e-5,
-                 seed: int = 0, max_ctas: int = 0, zero_init_residual: bool = True, native_stem: bool = True,
+                 seed: int = 0, max_ctas: int = 0, zero_init_residual: bool = True,
                  overlap_wgrad: bool = True, wgrad_smem_budget: int = 0, fuse_bwd_reduce: bool = True,
                  fuse_bn_coeffs: bool = False, fuse_block_grad: Optional[bool] = None,
                  fuse_stem_bwd: Optional[bool] = None):
+        if fuse_bn_coeffs:
+            raise ValueError("fuse_bn_coeffs was removed: BN coefficients inside the apply kernels measured slower "
+                             "(profiles/README.md, section 2.9)")
+        if fuse_stem_bwd:
+            raise ValueError("fuse_stem_bwd was removed: max-pool backward fused with the stem BN backward measured "
+                             "slower (profiles/README.md, R2.4)")
         ops.require_native()
         self.zero_init_residual = zero_init_residual
-        self.native_stem = native_stem
         # experimental: run every weight-gradient GEMM on a side stream so it overlaps the (DRAM-bound) BatchNorm
         # backward passes of the next layer; needs two dy scratch buffers and event-ordered buffer reuse
         self.overlap_wgrad = overlap_wgrad
         # BatchNorm-backward reductions of bn1/bn2 computed inside the dgrad GEMM that produces their input gradient
         self.fuse_bwd_reduce = fuse_bwd_reduce
-        # OPT-IN (B200DDL_FUSE_BN_COEFFS=1): BatchNorm scale/shift (forward) and A/B/C (backward) computed inside the apply
-        # kernels instead of 106 tiny launches.  Numerically equivalent (backward bit-identical), but MEASURED SLOWER:
-        # 19.39 vs 18.89 ms per step in an interleaved A/B at equal clocks (profiles/README.md 2.9) - a tiny dependent
-        # kernel costs only ~1.6 us of step time, the per-CTA coefficient recomputation in 106 streaming kernels more.
-        self.fuse_bn_coeffs = fuse_bn_coeffs or os.environ.get("B200DDL_FUSE_BN_COEFFS") == "1"
         # the gradient merge at every residual-block boundary (main path + skip path, ReLU mask, bn3 reduction) runs in
         # the epilogue of the next block's conv1 dgrad GEMM (conv_igemm kStats = 3); B200DDL_NO_BLOCK_GRAD=1 disables
         self.fuse_block_grad = (os.environ.get("B200DDL_NO_BLOCK_GRAD") != "1") if fuse_block_grad is None else bool(fuse_block_grad)
-        # max-pool backward fused with the stem BatchNorm backward (csrc/head_stem.cu); B200DDL_STEM_BWD_FUSE=1 enables
-        # MEASURED SLOWER in its first version (profiles/README.md r2: 1,162 vs 884 us per step at batch 256), so opt-in:
-        self.fuse_stem_bwd = (os.environ.get("B200DDL_STEM_BWD_FUSE") == "1") if fuse_stem_bwd is None else bool(fuse_stem_bwd)
+        self.fuse_stem_bwd = False  # reported by bench.py
         self._fused_reduce = set()
         self._block_fused = set()   # bn3 names whose reduction (and dz) come out of a fused dgrad epilogue
         # inference-only builds (build(training=False)): BatchNorm (running statistics) + ReLU + residual add run in the
-        # convolutions' epilogues (conv_igemm kStats = 4) - no BatchNorm pass at all.  B200DDL_NO_FUSED_INFER=1 disables.
-        self.fused_inference = os.environ.get("B200DDL_NO_FUSED_INFER") != "1"
+        # convolutions' epilogues (conv_igemm kStats = 4) - no BatchNorm pass at all.
         self._infer_fused = False
-        # OPT-IN (B200DDL_TAILS=1): BatchNorm finalize / backward-coefficient computation in the LAST CTA of the GEMM that
-        # accumulated the sums (conv_igemm last-CTA tails) instead of ~100 tiny dependent launches per step.  Numerically
-        # equivalent (gpu_check.py tails) but MEASURED SLOWER: 17.64 vs 17.11 ms per step, interleaved, both at 1965 MHz
-        # (profiles/r2_ab6_*.json): fence + ticket + a serial per-channel loop in ONE CTA at the end of every GEMM costs
-        # more than the ~4 us of a tiny dependent kernel that runs on all SMs.
-        self.fuse_tails = os.environ.get("B200DDL_TAILS") == "1" and not self.fuse_bn_coeffs
-        self._fin_fwd = set()    # BatchNorms finalized by their producing conv's tail (training mode)
-        self._fin_bwd = set()    # BatchNorms whose backward coefficients come from a dgrad tail
-        self._tail_plans = []
-        self._tail_state = None
         self.wgrad_smem_budget = wgrad_smem_budget
         self.aux_streams: List[torch.cuda.Stream] = []
         if image_size % 32:
@@ -253,13 +240,7 @@ class ResNet50Engine:
             self._bn_fwd(bn, 1.0, False)
 
     def _refresh_stem_weight(self) -> None:
-        if self.native_stem:
-            self._e.pack_stem_weight(self.p("conv1.weight"), self._stem_w16)
-        else:
-            self._stem_w.copy_(self._stem_oihw_from_flat())
-
-    def _stem_oihw_from_flat(self) -> torch.Tensor:
-        return self.p("conv1.weight").view(7, 7, 64, 3).permute(2, 3, 0, 1)
+        self._e.pack_stem_weight(self.p("conv1.weight"), self._stem_w16)
 
     # ------------------------------------------------------------------------------------------------ build
     def bind_grad_buffer(self, grads: Optional[torch.Tensor] = None) -> None:
@@ -285,7 +266,6 @@ class ResNet50Engine:
         S = self.image_size
         self.x_u8 = torch.zeros(N, S, S, 3, device=dev, dtype=torch.uint8)
         self.labels = torch.zeros(N, device=dev, dtype=torch.int64)
-        self.x16 = torch.zeros(N, S, S, 3, **bf)
         self.stats = torch.zeros(2, **f32)          # [sum loss, correct]
         self.logits = torch.zeros(N, self.num_classes, **f32)  # fp32 logits (+bias) for predict(); written by the CE kernel
         self.loss_rows = torch.zeros(N, **f32)
@@ -313,11 +293,8 @@ class ResNet50Engine:
         self.p0 = torch.zeros(N, H0 // 2, H0 // 2, 64, **bf)
         self.pool_idx = torch.zeros(N, H0 // 2, H0 // 2, 64, device=dev, dtype=torch.uint8)
         w0 = self.bnw["bn1"]
-        if self.native_stem:
-            self._stem_w16 = torch.zeros(64, 192, **bf)
-            self._stem_fwd = C.StemForward(self.x_u8, self._stem_w16, self.y0, w0["sum"], w0["sqsum"], max_ctas=self.max_ctas)
-        else:
-            self._stem_w = torch.zeros(64, 3, 7, 7, **bf).contiguous(memory_format=torch.channels_last)
+        self._stem_w16 = torch.zeros(64, 192, **bf)
+        self._stem_fwd = C.StemForward(self.x_u8, self._stem_w16, self.y0, w0["sum"], w0["sqsum"], max_ctas=self.max_ctas)
         self._refresh_stem_weight()
 
         max_act = N * (S // 4) * (S // 4) * 256
@@ -395,26 +372,7 @@ class ResNet50Engine:
 
         dz_keys = ["dzA", "dzB"]
         x_in = self.p0
-        self._infer_fused = (not training) and self.fused_inference
-        self._fin_fwd.clear()
-        self._fin_bwd.clear()
-        self._tail_plans = []
-        self._tail_state = None
-        tail_counters = torch.zeros(256, device=dev, dtype=torch.int32)
-        n_tail = [0]
-
-        def next_counter():
-            n_tail[0] += 1
-            return tail_counters[n_tail[0] - 1:n_tail[0]]
-
-        def bwd_tail(plan, bn_name: str, count: int) -> None:
-            """dgrad plan that reduces sum(dz), sum(dz*y) of `bn_name`: its last CTA also emits dgamma / dbeta / A, B, C."""
-            if not (self.fuse_tails and training):
-                return
-            w_ = self.bnw[bn_name]
-            plan.set_bn_bwd_coeffs(next_counter(), self.p(bn_name + ".weight"), w_["mean"], w_["invstd"], float(count),
-                                   self.g(bn_name + ".weight"), self.g(bn_name + ".bias"), w_["cA"], w_["cB"], w_["cC"])
-            self._fin_bwd.add(bn_name)
+        self._infer_fused = not training
         for bi, b in enumerate(self.blocks if self._infer_fused else []):
             # inference: every convolution writes its block activation directly (folded BN + ReLU [+ residual] epilogue)
             Hi, Ho, mid, cout = b.h_in, b.h_out, b.mid, b.mid * 4
@@ -467,15 +425,6 @@ class ResNet50Engine:
                 bw_ = self.bnw[b.name + "." + bnk]
                 y = A[b.name + "." + yk]
                 self._fwd[full] = C.ConvForward(xin, w2d, y, k, k, stride, pad, bw_["sum"], bw_["sqsum"], mc)
-                if training and self.fuse_tails:
-                    bname = b.name + "." + bnk
-                    cnt = N * y.shape[1] * y.shape[2]
-                    self._fwd[full].plan.set_bn_finalize(next_counter(), self.p(bname + ".weight"), self.p(bname + ".bias"),
-                                                         self.running_mean[bname], self.running_var[bname], bw_["mean"],
-                                                         bw_["invstd"], bw_["scale"], bw_["shift"], float(cnt),
-                                                         self.bn_momentum, self.bn_eps)
-                    self._fin_fwd.add(bname)
-                    self._tail_plans.append(self._fwd[full].plan)
                 if training:
                     dy = scr(self._dy_key[cname], y.shape)
                     gw = self.g(full + ".weight")
@@ -511,12 +460,6 @@ class ResNet50Engine:
                         self._fused_reduce.add(b.name + "." + pbn)
                     dgr = C.ConvDgrad(dy, self.p(full + ".weight"), dx, k, k, d_stride, pad, mc, wbufs=wd_views(full),
                                       bwd_stats=bwd_stats, block_grad=block_grad)
-                    if bwd_stats is not None:     # reduces bn1 (conv2's dgrad, count = conv1's output grid) or bn2 (conv3's)
-                        pbn = b.name + (".bn1" if cname == "conv2" else ".bn2")
-                        bwd_tail(dgr.parts[0][0], pbn, N * (Hi * Hi if cname == "conv2" else Ho * Ho))
-                    if block_grad is not None:    # reduces the previous block's bn3
-                        pb = self.blocks[bi - 1]
-                        bwd_tail(dgr.parts[0][0], pb.name + ".bn3", N * pb.h_out * pb.h_out)
                     self._dg[full] = dgr
                     self._dgrads.append(dgr)
             x_in = A[b.name + ".out"]
@@ -534,9 +477,8 @@ class ResNet50Engine:
                                       self.g("fc.weight"), 1, 1, 1, 0, 0, mc, 0)
             self._fc_dg = C.ConvDgrad(self.dlogits16.view(N, 1, 1, ncp), self.p("fc.weight").view(1, ncp, 2048),
                                       self.dpooled.view(N, 1, 1, 2048), 1, 1, 1, 0, mc, wbufs=wd_views("fc"))
-            if self.native_stem:
-                dy0 = self._scr["dzA"][:self.y0.numel()].view(self.y0.shape)
-                self._stem_wg = C.StemWgrad(self.x_u8, dy0, self.g("conv1.weight").view(-1), max_ctas=self.max_ctas)
+            dy0 = self._scr["dzA"][:self.y0.numel()].view(self.y0.shape)
+            self._stem_wg = C.StemWgrad(self.x_u8, dy0, self.g("conv1.weight").view(-1), max_ctas=self.max_ctas)
         self._training_built = training
         self._built = True
         self.sync_weights()
@@ -545,28 +487,15 @@ class ResNet50Engine:
     # ------------------------------------------------------------------------------------------------ forward
     def _bn_fwd(self, bn: str, count: float, training: bool) -> Dict[str, torch.Tensor]:
         w = self.bnw[bn]
-        if training and bn in self._fin_fwd:
-            return w  # finalized by the last CTA of the conv that produced the statistics
         self._e.bn_finalize(w["sum"], w["sqsum"], float(count), self.p(bn + ".weight"), self.p(bn + ".bias"),
                             self.running_mean[bn], self.running_var[bn], self.bn_momentum, self.bn_eps, w["mean"],
                             w["invstd"], w["scale"], w["shift"], training)
         return w
 
-    def _bn_pack(self, bn: str) -> List[torch.Tensor]:
-        """Tensors of one BatchNorm in the order csrc/ops_bind.cpp bn_apply_fused expects (parameter views are taken at
-        call time: the flat parameter buffer may have been moved into symmetric memory after build())."""
-        w = self.bnw[bn]
-        return [w["sum"], w["sqsum"], self.p(bn + ".weight"), self.p(bn + ".bias"), self.running_mean[bn],
-                self.running_var[bn], w["mean"], w["invstd"], w["scale"], w["shift"]]
-
     def _bn_apply(self, bn: str, count: float, training: bool, y, out, res=None, res_bn: Optional[str] = None,
                   mask=None) -> None:
-        """out = relu(BN(y) [+ res | + BN_res(res)]); the coefficient computation is fused into the kernel in training."""
+        """out = relu(BN(y) [+ res | + BN_res(res)])."""
         e = self._e
-        if training and self.fuse_bn_coeffs:
-            e.bn_apply_fused(y, self._bn_pack(bn), float(count), self.bn_momentum, self.bn_eps, res,
-                             self._bn_pack(res_bn) if res_bn is not None else None, out, True, mask)
-            return
         w = self._bn_fwd(bn, count, training)
         if res_bn is not None:
             wd = self._bn_fwd(res_bn, count, training)
@@ -578,22 +507,8 @@ class ResNet50Engine:
         """x_u8 / labels (static inputs) -> logits, loss stats.  All launches go to the current stream."""
         e, N, A = self._e, self.batch, self.act
         w0 = self.bnw["bn1"]
-        if self._tail_plans and self._tail_state != training:
-            # eval-mode forwards of a training engine must not update running statistics: the conv tails are switched off
-            # (host-side kernel parameter, captured by value in the train / eval CUDA graphs) and bn_finalize runs instead
-            for pl in self._tail_plans:
-                pl.enable_tail(bool(training))
-            self._tail_state = training
-        if training and self.fuse_bn_coeffs:
-            e.zero_(self._bn_fwd_sums)  # nobody zeroes them after use on the fused path
-        if self.native_stem:
-            # 7x7/2 stem on the tensor cores straight from the uint8 batch (normalisation + BN statistics fused)
-            self._stem_fwd.run()
-        else:
-            e.preprocess_u8(self.x_u8, self.x16, 1.0 / 127.5, -1.0)
-            y0 = torch.nn.functional.conv2d(self.x16.permute(0, 3, 1, 2), self._stem_w, stride=2, padding=3)
-            self.y0.copy_(y0.permute(0, 2, 3, 1))
-            e.channel_stats(self.y0, w0["sum"], w0["sqsum"])
+        # 7x7/2 stem on the tensor cores straight from the uint8 batch (normalisation + BN statistics fused)
+        self._stem_fwd.run()
         cnt0 = N * self.y0.shape[1] * self.y0.shape[2]
         self._bn_fwd("bn1", cnt0, training)
         # BN + ReLU + 3x3/2 max-pool in one pass (the 112x112 activation is never written)
@@ -660,15 +575,9 @@ class ResNet50Engine:
             e.bn_bwd_reduce(3, g1, None, None, y, None, None, None, w["sum_dz"], w["sum_dzy"])
         src = dz if mode == 1 else g1
         sc, sh = (w["scale"], w["shift"]) if mode == 2 else (None, None)
-        if self.fuse_bn_coeffs:
-            # A, B, C computed in the apply kernel's prologue; its first row-block writes dgamma / dbeta
-            e.bn_bwd_apply_fused(src, y, sc, sh, w["sum_dz"], w["sum_dzy"], self.p(bn + ".weight"), w["mean"],
-                                 w["invstd"], float(count), self.g(bn + ".weight"), self.g(bn + ".bias"), dy)
-        else:
-            if bn not in self._fin_bwd:  # otherwise the dgrad GEMM's last CTA already produced dgamma / dbeta / A, B, C
-                e.bn_bwd_coeffs(w["sum_dz"], w["sum_dzy"], self.p(bn + ".weight"), w["mean"], w["invstd"], float(count),
-                                self.g(bn + ".weight"), self.g(bn + ".bias"), w["cA"], w["cB"], w["cC"])
-            e.bn_bwd_apply(src, y, sc, sh, w["cA"], w["cB"], w["cC"], dy)
+        e.bn_bwd_coeffs(w["sum_dz"], w["sum_dzy"], self.p(bn + ".weight"), w["mean"], w["invstd"], float(count),
+                        self.g(bn + ".weight"), self.g(bn + ".bias"), w["cA"], w["cB"], w["cC"])
+        e.bn_bwd_apply(src, y, sc, sh, w["cA"], w["cB"], w["cC"], dy)
         self._ready(bn + ".weight", bn + ".bias")
 
     def _dy_buf(self, cname: str, shape) -> torch.Tensor:
@@ -702,8 +611,6 @@ class ResNet50Engine:
         """dlogits -> every parameter gradient (fp32, written into the flat gradient buffer)."""
         e, N, A = self._e, self.batch, self.act
         e.zero_(self.grads)  # wgrad accumulates with atomics
-        if self.fuse_bn_coeffs:
-            e.zero_(self._bn_bwd_sums)  # sum(dz), sum(dz*y) of every layer; nobody zeroes them after use on the fused path
         # classifier head: wgrad + dgrad on the tcgen05 GEMMs, bias gradient = column sums of dlogits
         self._fc_wg.run()
         e.fc_bias_grad(self.dlogits16, self.g("fc.bias"))
@@ -755,26 +662,10 @@ class ResNet50Engine:
         # stem: g1 (main path of layer1.0) + g2 (its projection shortcut) flow through max-pool, ReLU and bn1
         dy0 = self._scr["dzA"][:self.y0.numel()].view(self.y0.shape)
         cnt0 = N * self.y0.shape[1] * self.y0.shape[2]
-        w0 = self.bnw["bn1"]
-        if self.fuse_stem_bwd and not self.fuse_bn_coeffs:
-            # max-pool backward + BN(+ReLU) backward without materialising the 112x112 pooled gradient
-            e.stem_pool_bn_bwd(0, self.pool_idx, g1, g2, self.y0, w0["scale"], w0["shift"], None, None, None, None,
-                               w0["sum_dz"], w0["sum_dzy"])
-            e.bn_bwd_coeffs(w0["sum_dz"], w0["sum_dzy"], self.p("bn1.weight"), w0["mean"], w0["invstd"], float(cnt0),
-                            self.g("bn1.weight"), self.g("bn1.bias"), w0["cA"], w0["cB"], w0["cC"])
-            e.stem_pool_bn_bwd(1, self.pool_idx, g1, g2, self.y0, w0["scale"], w0["shift"], w0["cA"], w0["cB"],
-                               w0["cC"], dy0, w0["sum_dz"], w0["sum_dzy"])
-            self._ready("bn1.weight", "bn1.bias")
-        else:
-            da0 = self._dy_buf("conv3", self.y0.shape)  # reuses the (by now idle) "dy" scratch
-            e.maxpool_bwd(self.pool_idx, g1, g2, da0)
-            self._bn_bwd("bn1", 2, da0, None, None, self.y0, dy0, None, cnt0)
-        if self.native_stem:
-            self._stem_wg.run()
-        else:
-            gw = torch.nn.grad.conv2d_weight(self.x16.permute(0, 3, 1, 2), (64, 3, 7, 7), dy0.permute(0, 3, 1, 2),
-                                             stride=2, padding=3)
-            self.g("conv1.weight").view(7, 7, 64, 3).copy_(gw.permute(2, 3, 0, 1))
+        da0 = self._dy_buf("conv3", self.y0.shape)  # reuses the (by now idle) "dy" scratch
+        e.maxpool_bwd(self.pool_idx, g1, g2, da0)
+        self._bn_bwd("bn1", 2, da0, None, None, self.y0, dy0, None, cnt0)
+        self._stem_wg.run()
         self._ready("conv1.weight")
         if self.overlap_wgrad:
             torch.cuda.current_stream().wait_stream(self._wg_stream)

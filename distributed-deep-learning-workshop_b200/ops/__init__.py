@@ -18,19 +18,8 @@ from . import _build
 EXT_NAMES = tuple(_build.EXTENSIONS)
 
 
-# Rows per loop iteration of the BatchNorm apply / backward-apply kernels (csrc/elementwise.cu): 1, 2 or 4, bit-identical
-# results; the default is the value the A/B in profiles/README.md R2.9 settled on, `B200DDL_BN_UNROLL` overrides it.
-BN_ROWS_UNROLL_DEFAULT = 1
-
-
 def ext(name: str):
-    fresh = name not in _build._loaded
-    mod = _build.load(name)
-    if fresh and name == "_b200_ops" and hasattr(mod, "set_bn_rows_unroll"):
-        import os
-
-        mod.set_bn_rows_unroll(int(os.environ.get("B200DDL_BN_UNROLL", BN_ROWS_UNROLL_DEFAULT)))
-    return mod
+    return _build.load(name)
 
 
 def build_all(verbose: bool = False) -> None:

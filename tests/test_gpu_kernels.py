@@ -67,11 +67,6 @@ def test_classifier_head_on_tcgen05(checks):
     assert checks.case_head()
 
 
-def test_stem_tail_backward_fused(checks):
-    """max-pool backward fused with the stem BN backward == the three-kernel path, bit for bit."""
-    assert checks.case_stem_bwd()
-
-
 def test_inference_epilogue_and_fused_inference_engine(checks):
     """conv epilogue with folded BatchNorm + activation (+ residual) vs fp32; inference-built engine vs eval on the training build."""
     assert checks.case_fused_infer()
@@ -80,17 +75,6 @@ def test_inference_epilogue_and_fused_inference_engine(checks):
 def test_reference_model_mobilenetv2_on_native_kernels(checks):
     """Frozen MobileNetV2 base + Dense head: depthwise / stem kernels and the whole engine vs the torch.nn module."""
     assert checks.case_mobilenet()
-
-
-def test_last_cta_batchnorm_tails(checks):
-    """BatchNorm finalize / backward coefficients computed by the last CTA of the GEMM that accumulated the sums."""
-    assert checks.case_tails()
-
-
-def test_resnet50_engine_with_last_cta_tails_matches_torchvision(checks, monkeypatch):
-    """Opt-in path (B200DDL_TAILS=1): BatchNorm finalize / backward coefficients in the GEMMs' last CTAs."""
-    monkeypatch.setenv("B200DDL_TAILS", "1")
-    assert checks.case_engine(quick=True)
 
 
 def test_conv_numerics_at_benchmark_batch(checks):
@@ -105,11 +89,6 @@ def test_resnet50_engine_unfused_block_gradient_matches_torchvision(checks):
 
 def test_resnet50_engine_matches_torchvision(checks):
     assert checks.case_engine()
-
-
-def test_resnet50_engine_fused_bn_coefficients_matches_torchvision(checks):
-    """Opt-in path: BatchNorm coefficients computed inside the apply kernels (same gradient criteria)."""
-    assert checks.case_engine(quick=True, fuse_bn_coeffs=True)
 
 
 def test_resnet50_engine_inline_wgrad_matches_torchvision(checks):
